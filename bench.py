@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR     (also writes the last timed step's results, see dump_outputs)
 
 Metric (BASELINE.json): sample-genotype calls per second (one call = one (sample, site) genotype call).
 Workload at N=1 (config.workload): BASELINE.json configs[2] "C3" -- 2,504 samples (1000G-shaped), 2-5 alleles per
@@ -36,10 +37,16 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (no __pycache__ of the modules it imports)
 
 METRIC = "sample_genotype_calls_per_s"
 UNIT = "calls/s"
 WORKLOAD = "C3"
+# --dump-outputs: at most 65,536 sites (every site of the default step) with their per-site fields, 128 of them with their
+# per-sample outputs (GT, GQ, PL); at 2,504 samples that is at most ~56 MB of float64 whatever --sites / --replicate are
+DUMP_SITES = 65536
+DUMP_SAMPLE_SITES = 128
+DUMP_SEED = 0xB200D
 
 
 def measured_peak():
@@ -241,6 +248,49 @@ def ncu_traffic(sites_per_step):
     return {int(k): int(v["dram_bytes_read"] + v["dram_bytes_write"]) for k, v in d.get("classes", {}).items()}, d.get("source", path)
 
 
+def dump_outputs(out_dir, db, dr):
+    """--dump-outputs DIR: the mcb_result arrays of the last timed step as DIR/<name>.npy, so that two builds can be compared
+    output for output (the inputs are seeded: the same arguments give the same step).  Site indices are step-wide.
+      sites [n]: every site of the step, or a fixed seeded sample of DUMP_SITES of them in a larger step; for these sites
+        ret, als_new, site_flags, an, qual [n]; als_map, ac [n, max_nals]; diag [n, 4]
+      sample_sites [k]: a fixed seeded sample of DUMP_SAMPLE_SITES of them; for these sites gt [k, nsmpl, 2], gq [k, nsmpl],
+        and their trimmed PL blocks concatenated in pl, the block of sample site j at pl[pl_site_offsets[j]:pl_site_offsets[j+1]]
+        ([nsmpl][G'] row-major; empty where ret <= 0 or the PLs were dropped)
+    qual is float32 as computed; every integer array is widened to float64, exact (the INT32 missing / vector-end sentinels
+    stay distinct)."""
+    import torch
+    from bcftools_b200 import abi
+    t, R, S = dr.t, db.nsites, db.nsmpl
+    rng = np.random.default_rng(DUMP_SEED)
+    sites = np.arange(R) if R <= DUMP_SITES else np.sort(rng.choice(R, size=DUMP_SITES, replace=False))
+    smp = np.sort(rng.choice(sites, size=min(DUMP_SAMPLE_SITES, sites.size), replace=False))
+    dev = t["gt"].device
+    out = dict(sites=sites, sample_sites=smp)
+    for name in ("ret", "als_new", "als_map", "qual", "ac", "an", "site_flags", "diag"):
+        out[name] = t[name].index_select(0, torch.from_numpy(sites).to(dev)).cpu().numpy().view(abi.RESULT_FIELDS[name])
+    for name in ("gt", "gq"):
+        if t[name] is not None:
+            out[name] = t[name].index_select(0, torch.from_numpy(smp).to(dev)).cpu().numpy()
+    ret = t["ret"].cpu().numpy()
+    flags = t["site_flags"].cpu().numpy().view(np.uint32)
+    blocks, offs = [], [0]
+    for i in smp:
+        n = int(ret[i])
+        g = S * n * (n + 1) // 2 if n > 0 and not (flags[i] & abi.SITE_PL_DROPPED) else 0
+        o = int(db.pl_off_host[i])
+        blocks.append(t["pl"][o:o + g].cpu().numpy())
+        offs.append(offs[-1] + g)
+    out["pl"] = np.concatenate(blocks)
+    out["pl_site_offsets"] = np.array(offs)
+    out = {name: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64) for name, a in out.items()}
+    total = sum(a.nbytes for a in out.values())
+    assert total <= 64_000_000, total
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -258,7 +308,13 @@ def main():
     ap.add_argument("--job-sites-per-gpu", type=int, default=192, help="N>1: C4-shaped sites per GPU of the one-job strong-scaling leg (rank 0 drives all N GPUs)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step of rank 0 as DIR/<name>.npy "
+                                                          "(the CUDA path only: not with --impl reference)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the results of the CUDA path: not with --impl reference")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -312,6 +368,8 @@ def main():
     barrier()
     dev_s = e0.elapsed_time(e1) * 1e-3
     launches = int(mc.stats()[0]) * args.steps
+    # the legs below reuse the result buffers: the outputs of the timed steps are taken now
+    dumped_bytes = dump_outputs(args.dump_outputs, db, dr) if args.dump_outputs and rank == 0 else None
     # ---- sustained leg: the timed region above lasts ~50 ms at boost clocks; these kernels are issue-bound, so a long job
     # runs at whatever clock the power limit settles on.  Same step, >= --sustain seconds, its own clock samples.
     sustained = None
@@ -533,7 +591,8 @@ def main():
                                 l2_policy="inputs larger than L2 (%.2f GB of PL per step)" % (db.pl_bytes() / 1e9),
                                 bytes_per_call=(rd_all + wr_all) / (hb.nsites * params.nsmpl), generator_version=synth.GENERATOR_VERSION),
                     gpu_launches=launches, clocks=sampler.summary(), roofline=roof, cpu_baseline=cpu, e2e=e2e, parity=parity,
-                    sustained=sustained, secondary=secondary, job=job)
+                    sustained=sustained, secondary=secondary, job=job,
+                    dumped_outputs=None if dumped_bytes is None else dict(dir=args.dump_outputs, bytes=dumped_bytes))
         print(json.dumps(line, default=lambda o: o.item() if hasattr(o, 'item') else str(o)), flush=True)
     if world > 1:
         dist.destroy_process_group()

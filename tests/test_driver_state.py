@@ -1,6 +1,7 @@
 """include/b200_driver.h (SURVEY.md 8f N2): ploidy definitions + set_ploidy, -G group files, the unseen allele -- against
 the committed golden cases (whose per-site ploidy vectors / unseen alleles / groups reproduce the reference's outputs),
-the reference's own option files where the reference tree is present, and the quirks of ploidy.c / mcall.c."""
+the reference's own option files and expected outputs (bundled in tests/golden/vcf_text_cases.json.gz), its ploidy
+presets (tests/golden/ploidy_presets.txt) and the quirks of ploidy.c / mcall.c."""
 import os
 import re
 
@@ -8,10 +9,14 @@ import numpy as np
 import pytest
 
 from bcftools_b200 import driver
-from tests import golden_util
+from tests import golden_util, vcf_cases
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF_TEST = "/root/reference/test"
+
+
+def _ref_file(name):
+    """Text of a file of the reference's test/ directory, from the committed bundle."""
+    return vcf_cases.bundle()["files"][name]
 
 # the definition the reference's chrX tests use (test/test.pl:281-283), in the format of ploidy.c:40-53
 PLOIDY_X = "X 1 1000 M 1\nX 3104 5000 M 1\n* * * M 2\n* * * F 2\n"
@@ -104,12 +109,9 @@ def test_groups_parse_semantics():
 @pytest.mark.parametrize("name,fname", [("call.af-fixation.2", "call.af-fixation.txt"), ("mpileup.hwe.4", "mpileup.hwe.samples")])
 def test_groups_of_the_reference_option_files(name, fname):
     """The reference's own -G files (test/test.pl:287, 306): the parsed member lists must be the groups the golden case
-    was generated with.  Needs the reference tree (this container); skipped elsewhere."""
-    path = os.path.join(REF_TEST, fname)
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
+    was generated with."""
     case = golden_util.load_case(name)[3]
-    off, g = driver.groups_parse(open(path).read(), case["samples"])
+    off, g = driver.groups_parse(_ref_file(fname), case["samples"])
     got = [g[off[k]:off[k + 1]].tolist() for k in range(len(off) - 1)]
     assert got == case["groups"]
 
@@ -148,13 +150,10 @@ def test_samples_parse_semantics():
                                         ("mpileup.X", "mpileup.samples"), ("mpileup.X.ped", "mpileup.ped"), ("mpileup.X.2", "mpileup.2.samples")])
 def test_samples_of_the_reference_option_files(name, fname):
     """The reference's own -S files (test/test.pl:278-283): selected samples in the order of the golden case, and -- with the
-    chrX ploidy definition -- the per-site ploidy vectors of the golden via set_ploidy.  Needs the reference tree."""
-    path = os.path.join(REF_TEST, fname)
-    if not os.path.exists(path):
-        pytest.skip("reference tree not present")
+    chrX ploidy definition -- the per-site ploidy vectors of the golden via set_ploidy."""
     case = golden_util.load_case(name)[3]
     pl = driver.Ploidy(PLOIDY_X if "X" in name else "* * * M 2\n* * * F 2\n", 2)
-    smap, s2s, warn = pl.samples_parse(open(path).read(), HDR3)
+    smap, s2s, warn = pl.samples_parse(_ref_file(fname), HDR3)
     assert [HDR3[m] for m in smap] == case["samples"]
     prev = np.full(len(pl.sexes), pl.max(), np.int32)
     ploidy = np.full(len(smap), pl.max(), np.uint8)
@@ -164,9 +163,9 @@ def test_samples_of_the_reference_option_files(name, fname):
     pl.close()
 
 
-def _vcf_records(path):
+def _vcf_records(text):
     out = []
-    for l in open(path):
+    for l in text.splitlines(True):
         if l.startswith("#"):
             continue
         f = l.rstrip("\n").split("\t")
@@ -187,12 +186,10 @@ def test_trim_numberR_semantics():
                                      ("mpileup.hwe.vcf", "mpileup.hwe.2.out"), ("call.af-fixation.vcf", "call.af-fixation.1.out")])
 def test_finaliser_pieces_against_the_reference_outputs(vcf, out):
     """DP4 / MQ from INFO/I16 (mcall.c:1660-1666) and the Number=R trimming of FORMAT/AD (mcall.c:1196-1265) against the records
-    of the reference's own expected outputs.  Needs the reference tree (this container); skipped elsewhere."""
-    if not os.path.exists(os.path.join(REF_TEST, vcf)):
-        pytest.skip("reference tree not present")
-    src = {(r["chrom"], r["pos"], r["ref"]): r for r in _vcf_records(os.path.join(REF_TEST, vcf))}
+    of the reference's own expected outputs."""
+    src = {(r["chrom"], r["pos"], r["ref"]): r for r in _vcf_records(_ref_file(vcf))}
     n_dp4 = n_ad = 0
-    for o in _vcf_records(os.path.join(REF_TEST, out)):
+    for o in _vcf_records(_ref_file(out)):
         r = src.get((o["chrom"], o["pos"], o["ref"]))
         if r is None or "I16" not in r["info"]:
             continue
@@ -232,15 +229,11 @@ def test_ploidy_aliases():
 
 
 def test_ploidy_aliases_against_the_reference_source():
-    """Every preset of vcfcall.c:138-198, parsed out of the reference source where the tree is present, answers the same
-    per-sex ploidies as the alias on a grid of positions around all of its region boundaries."""
-    src = "/root/reference/vcfcall.c"
-    if not os.path.exists(src):
-        pytest.skip("reference tree not present")
-    text = open(src).read()
+    """Every preset of vcfcall.c:138-198 (its .ploidy strings, kept in tests/golden/ploidy_presets.txt under one '# alias'
+    line each) answers the same per-sex ploidies as the alias on a grid of positions around all of its region boundaries."""
+    text = open(os.path.join(ROOT, "tests", "golden", "ploidy_presets.txt")).read()
     n = 0
-    for m in re.finditer(r'\.alias\s*=\s*"([^"]+)".*?\.ploidy\s*=\s*((?:\s*"[^"]*"\s*)+)', text, flags=re.S):
-        alias, body = m.group(1), "".join(re.findall(r'"([^"]*)"', m.group(2))).replace("\\n", "\n")
+    for alias, body in re.findall(r"^# (\S+)\n((?:[^#].*\n)+)", text, flags=re.M):
         ref, mine = driver.Ploidy(body, 2), driver.Ploidy(alias=alias)
         assert ref.sexes == mine.sexes, alias
         probes = [("7", 100)]
