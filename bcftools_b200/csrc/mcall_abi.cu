@@ -83,6 +83,7 @@ struct mcb_ctx
     int64_t opt_mm_block = 0;            /* its CTA size (0 = automatic) */
     int64_t opt_mm_block_c[NCLASS] = {0,0,0,0,0,0};     /* ... per allele-count class */
     int64_t opt_warp2 = -1;              /* biallelic warp-per-site kernel: -1 automatic, 0 off, n = force n warps per CTA */
+    int64_t opt_warp3 = -1;              /* 3-allele warp-per-site kernel: -1 automatic, 0 off, n = at most n warps per CTA */
     int64_t opt_order = 54321;           /* launch order of the allele-count classes */
     int64_t opt_time_kernels = 0, opt_concurrent = 1;    /* class kernels on their own streams: a class fills the tail of the previous one (-3.5 % per C3 step) */
     int64_t opt_ring_bytes_c[NCLASS] = {0,0,0,0,0,0};   /* per allele-count class override of ring_bytes (0 = opt_ring_bytes) */
@@ -198,6 +199,7 @@ extern "C" int mcb_set_option(mcb_ctx *ctx, const char *key, int64_t value)
     else if ( !strcmp(key,"mm_block") )      { if ( value!=0 && value!=64 && value!=128 && value!=256 ) return MCB_EINVAL; ctx->opt_mm_block = value; }
     else if ( !strncmp(key,"mm_block_",9) && key[9]>='3' && key[9]<='5' && !key[10] ) { if ( value!=0 && value!=64 && value!=128 && value!=256 ) return MCB_EINVAL; ctx->opt_mm_block_c[key[9]-'0'] = value; }
     else if ( !strcmp(key,"warp2") )         { if ( value<-1 || value>biallelic_max_warps() ) return MCB_EINVAL; ctx->opt_warp2 = value; }
+    else if ( !strcmp(key,"warp3") )         { if ( value<-1 || value>triallelic_max_warps() ) return MCB_EINVAL; ctx->opt_warp3 = value; }
     else if ( !strncmp(key,"ring_bytes_",11) && key[11]>='1' && key[11]<='5' && !key[12] ) ctx->opt_ring_bytes_c[key[11]-'0'] = value;
     else if ( !strncmp(key,"block_",6) && key[6]>='1' && key[6]<='5' && !key[7] )
     {
@@ -366,6 +368,17 @@ extern "C" int mcb_get_kernel_times(mcb_ctx *ctx, float ms[6])
     CK(cudaEventSynchronize(ctx->kev[5]));
     ms[0] = 0;
     for (int k=1; k<=5; k++) { CK(cudaEventElapsedTime(&ms[k], ctx->kev[k-1], ctx->kev[k])); ms[0] += ms[k]; }
+    return MCB_OK;
+}
+
+/*  Sites of each allele-count class (n[k], k=3..5; the other entries are 0) that the multi-allelic kernels of the last
+ *  mcb_call_device handed back to the general kernel through their fallback lists (synchronises the device).              */
+extern "C" int mcb_get_fallback_counts(mcb_ctx *ctx, int32_t n[6])
+{
+    if ( !ctx || !n || !ctx->d_counts ) return MCB_EINVAL;
+    CK(cudaSetDevice(ctx->device));
+    CK(cudaDeviceSynchronize());
+    CK(cudaMemcpy(n, ctx->d_counts + NCLASS + 8, sizeof(int32_t)*6, cudaMemcpyDeviceToHost));
     return MCB_OK;
 }
 
@@ -633,11 +646,45 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
         int grid = (int)std::min<int64_t>((int64_t)b->nsites, (int64_t)ctx->nsm*nb);
         cudaStream_t cs = fork ? ctx->cstream[nals] : st;
         if ( fork ) CK(cudaStreamWaitEvent(cs, ctx->cev_fork, 0));
-        /*  3-5 alleles, int32 PLs, every sample diploid, GT + GQ + PL requested: the CTA-per-site kernel of mcall_multi.cu.
-         *  Sites it has no straight-line code for come back on a fallback list, which the general kernel below walks.  */
-        if ( nals>=3 && ctx->opt_multi && !ctx->opt_exact && !ctx->opt_block && !ctx->opt_block_c[nals] && pl_es==4 && !ploidy && !gpk && a.gt && a.gq && a.out_pl && !(a.flag & MCB_CALL_KEEPALT)
+        /*  3-5 alleles, int32 PLs, every sample diploid, GT + GQ + PL requested: the CTA-per-site kernel of mcall_multi.cu, or for
+         *  3 alleles the warp-per-site kernel of mcall_triallelic.cu.  Sites they have no straight-line code for come back on a
+         *  fallback list, which the general kernel below walks.  */
+        const bool multi_ok = nals>=3 && ctx->opt_multi && !ctx->opt_exact && !ctx->opt_block && !ctx->opt_block_c[nals] && pl_es==4 && !ploidy && !gpk && a.gt && a.gq && a.out_pl && !(a.flag & MCB_CALL_KEEPALT)
              && (a.output_tags & (MCB_CALL_FMT_GQ|MCB_CALL_FMT_GP))
-             && !((reinterpret_cast<uintptr_t>(a.gt) | reinterpret_cast<uintptr_t>(a.gq) | reinterpret_cast<uintptr_t>(a.out_pl)) & 15) )
+             && !((reinterpret_cast<uintptr_t>(a.gt) | reinterpret_cast<uintptr_t>(a.gq) | reinterpret_cast<uintptr_t>(a.out_pl)) & 15);
+        int tw_warps = 0;
+        if ( multi_ok && nals==3 && ctx->opt_warp3!=0 && multi_block_for(a.nsmpl) )
+        {
+            const int ncta = triallelic_ctas_per_sm();
+            const size_t per_cta = (size_t)(ctx->smem_per_sm/ncta) - 1024;  /* the kernel is compiled for ncta CTAs per SM */
+            int w = triallelic_max_warps();
+            while ( w>0 && triallelic_smem_bytes(a.nsmpl, w) > per_cta ) w--;
+            if ( ctx->opt_warp3>0 ) w = std::min<int>(w, (int)ctx->opt_warp3);
+            /* an explicit CTA size or ring depth of the class asks for the CTA kernel; below 12 resident warps per SM it wins */
+            const bool cta_forced = ctx->opt_mm_block || ctx->opt_mm_block_c[3] || ctx->opt_mm_nst || ctx->opt_mm_nst_c[3];
+            if ( ctx->opt_warp3>0 ? w>0 : (w*ncta>=12 && !cta_forced) ) tw_warps = w;
+        }
+        if ( tw_warps )
+        {
+            const int tgrid = (int)std::min<int64_t>(((int64_t)b->nsites + tw_warps - 1)/tw_warps, (int64_t)ctx->nsm*triallelic_ctas_per_sm());
+            KArgs am = a;
+            am.fb_list = lists + (size_t)(NCLASS + nals)*list_stride;
+            am.fb_count = counts + NCLASS + 8 + nals;
+            cudaError_t le = launch_triallelic_warp_kernel(am, tgrid, tw_warps, cs);
+            if ( le==cudaSuccess && getenv("MCB_DEBUG_SYNC") ) le = cudaStreamSynchronize(cs);
+            if ( le!=cudaSuccess )
+            {
+                char what[160];
+                snprintf(what, sizeof what, "3-allele warp kernel warps=%d grid=%d smem=%zu", tw_warps, tgrid, triallelic_smem_bytes(a.nsmpl, tw_warps));
+                return cuda_fail(ctx, le, what);
+            }
+            launches++;
+            /* the general kernel now walks the fallback list only */
+            a.site_list = am.fb_list; a.site_count = am.fb_count;
+            a.work_counter = counts + NCLASS + 16 + nals;
+            grid = std::min(grid, ctx->nsm);
+        }
+        else if ( multi_ok )
         {
             /* CTA size: explicit option, else the class default (sweeps in profiles/), never below what the 12-bit allele counters allow */
             const int minblock = multi_block_for(a.nsmpl);

@@ -64,13 +64,6 @@ struct BWRec                            /* written by lane 0 after phase 1, read
 static_assert(sizeof(BWRec) <= BW_REC_BYTES, "BWRec grew past its slot");
 static_assert(offsetof(BWRec, scr_w) % 16 == 0, "scr_w is read with one 128-bit load");
 
-struct BWTables
-{
-    double pl2p[256];
-    double gq_thr[130];
-    ScreenTabs scr;                     /* float32 screen of phase 2 (mcall_device.cuh) */
-};
-
 /*  the literal FP64 call of one diploid sample of a pair site from its packed bytes: the samples the float32 screen does not accept  */
 static __device__ __noinline__ int bw_fast2_exact(uint32_t a, uint32_t b, uint32_t c, double q0, double q1, uint32_t pl2p_s, uint32_t thr_s)      /* slot | GQ << 8 */
 {

@@ -91,6 +91,11 @@ size_t multi_smem_bytes(int nals, int block, int nsmpl, int nst);
 size_t multi_scratch_bytes(int nsmpl, int grid);
 cudaError_t multi_kernel_occupancy(int nals, int block, int nsmpl, int nst, int *blocks_per_sm);
 cudaError_t launch_multi_kernel(int nals, int block, const KArgs &a, int grid, cudaStream_t st);
+/*  warp-per-site kernel of the 3-allele class over the same packed copy (mcall_triallelic.cu)  */
+size_t triallelic_smem_bytes(int nsmpl, int nwarp);
+int triallelic_max_warps();
+int triallelic_ctas_per_sm();
+cudaError_t launch_triallelic_warp_kernel(const KArgs &a, int grid, int nwarp, cudaStream_t st);
 /*  warp-per-site kernel for grouped calling (-G) of two-allele sites (mcall_biallelic_groups.cu)  */
 bool biallelic_groups_ok(int nsmpl, int ngroups);
 int biallelic_groups_warps();

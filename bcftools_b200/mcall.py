@@ -16,7 +16,7 @@ _lib = None
 
 EXPORTS = ["mcb_init", "mcb_destroy", "mcb_set_ploidy", "mcb_call_device", "mcb_call_host", "mcb_host_alloc",
            "mcb_host_free", "mcb_strerror", "mcb_last_cuda_error", "mcb_get_theta", "mcb_get_pl2p", "mcb_get_stats",
-           "mcb_set_option", "mcb_version", "mcb_selftest_div", "mcb_get_kernel_times"]
+           "mcb_set_option", "mcb_version", "mcb_selftest_div", "mcb_get_kernel_times", "mcb_get_fallback_counts"]
 
 
 JOB_EXPORTS = ["mcb_job_init", "mcb_job_destroy", "mcb_job_ndevices", "mcb_job_set_ploidy", "mcb_job_set_option",
@@ -65,6 +65,8 @@ def lib():
         L.mcb_version.restype = C.c_int
         L.mcb_get_kernel_times.restype = C.c_int
         L.mcb_get_kernel_times.argtypes = [C.c_void_p, C.c_void_p]
+        L.mcb_get_fallback_counts.restype = C.c_int
+        L.mcb_get_fallback_counts.argtypes = [C.c_void_p, C.c_void_p]
         L.mcb_selftest_div.restype = C.c_int
         L.mcb_selftest_div.argtypes = [C.c_void_p, C.c_int, C.c_uint64, C.c_uint64, C.POINTER(C.c_uint64)]
         L.mcb_job_init.restype = C.c_int
@@ -249,6 +251,12 @@ class MCaller:
         """Per allele-count class device time of the last call_device (option time_kernels=1): array[6], [0]=sum."""
         out = np.zeros(6, np.float32)
         self._check(lib().mcb_get_kernel_times(self._ctx, out.ctypes.data), "mcb_get_kernel_times")
+        return out
+
+    def fallback_counts(self):
+        """Sites per allele-count class that the multi-allelic kernels of the last call_device handed to the general kernel: array[6]."""
+        out = np.zeros(6, np.int32)
+        self._check(lib().mcb_get_fallback_counts(self._ctx, out.ctypes.data), "mcb_get_fallback_counts")
         return out
 
     def selftest_div(self, mode, n=0, seed=1):

@@ -188,6 +188,9 @@ int   mcb_version(void);
 /*  device milliseconds of the site kernel per allele-count class (ms[1..5], ms[0]=sum) of the last
  *  mcb_call_device; requires mcb_set_option(ctx,"time_kernels",1) */
 int   mcb_get_kernel_times(mcb_ctx *ctx, float ms[6]);
+/*  sites of each allele-count class (n[3..5]) that the multi-allelic kernels of the last mcb_call_device handed back to the
+ *  general kernel (DESIGN.md 4b); synchronises the device  */
+int   mcb_get_fallback_counts(mcb_ctx *ctx, int32_t n[6]);
 /*  device self-test of the shared-reciprocal IEEE division (mode 0: exhaustive 256^3 biallelic domain;
  *  mode 6/10/15: n random vectors of that many genotypes); *mismatch must come back 0 */
 int   mcb_selftest_div(mcb_ctx *ctx, int mode, uint64_t n, uint64_t seed, uint64_t *mismatch);
