@@ -24,6 +24,7 @@ SITE_UNSEEN_SEL = 1 << 2
 SITE_TOO_MANY_ALS = 1 << 3
 SITE_NO_QS = 1 << 4
 SITE_REF_GT = 1 << 5
+SITE_ADJUDICATED = 1 << 9        # near tie evaluated again with the literal phase 1 (option "adjudicate"); with SITE_NEAR_TIE
 
 MCB_OK, MCB_EINVAL, MCB_ENOMEM, MCB_ECUDA, MCB_ENODEV, MCB_EPL, MCB_EQS, MCB_EPRIOR = 0, -1, -2, -3, -4, -5, -6, -7
 

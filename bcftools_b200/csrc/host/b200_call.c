@@ -27,10 +27,6 @@ typedef struct
     void **user_out;
     int nres;
     int ploidy_upto;        /* ploidy ids below this must be registered with the context before the batch runs */
-    /* near-tie adjudication: sites that came back with MCB_SITE_NEAR_TIE were run a second time with the literal phase 1;
-       adj_idx[i] >= 0: record i is served from entry adj_idx[i] of `adj` (trimmed PL / GP at adj_pl_off[]) */
-    int *adj_idx;  int adj_n, adj_cap;  int64_t adj_pl_cap;
-    mcb_batch adj_in;  mcb_result adj;  int64_t *adj_pl_off;
 }
 b200_slabs_t;
 
@@ -82,67 +78,6 @@ static void *xcalloc(size_t n, size_t size)
     return p;
 }
 
-#define MCB_SITE_ADJUDICATED (1u<<9)     /* re-evaluated with the literal phase 1 (mcb_set_option exact_phase1) */
-#define REGROW(ptr, type, n) do { free(ptr); (ptr) = (type*) xcalloc((size_t)(n), sizeof(type)); } while (0)
-
-/*  The sites of the batch whose two best allele sets are closer than tie_eps are called a second time with
- *  mcb_set_option(ctx, "exact_phase1", 1): the device then sums log(val) sample by sample in the reference's order
- *  (mcall.c:607-611, 635-645, 680-690) instead of multiplying, so the choice between the two sets is the reference's
- *  up to the last bit of log() itself.  Pooled calling with int32 PLs; grouped and typed batches keep the flag only.  */
-static int adjudicate(b200_batcher_t *b, b200_slabs_t *s, int want_gq, char *err, size_t nerr)
-{
-    const int S = b->nsmpl, M = b->max_nals;
-    int n = 0;
-    for (int i=0; i<s->n; i++) { s->adj_idx[i] = -1; if ( s->res.site_flags[i] & MCB_SITE_NEAR_TIE ) n++; }
-    s->adj_n = 0;
-    if ( !n ) return 0;
-    int64_t pl_need = 0;
-    for (int i=0; i<s->n; i++)
-        if ( s->res.site_flags[i] & MCB_SITE_NEAR_TIE ) pl_need += (((int64_t)S*s->nals[i]*(s->nals[i]+1)/2) + 3) & ~(int64_t)3;
-    mcb_batch *in = &s->adj_in; mcb_result *r = &s->adj;
-    if ( n > s->adj_cap )
-    {
-        s->adj_cap = n;
-        REGROW(in->pl_off, int64_t, n); REGROW(in->nals, uint8_t, n); REGROW(in->unseen, uint8_t, n); REGROW(in->nqs, uint8_t, n);
-        REGROW(in->ploidy_id, uint16_t, n); REGROW(in->qs, float, (size_t)n*M); REGROW(in->prior_an, int32_t, n); REGROW(in->prior_ac, int32_t, (size_t)n*M);
-        REGROW(r->ret, int32_t, n); REGROW(r->als_new, uint32_t, n); REGROW(r->als_map, int8_t, (size_t)n*M); REGROW(r->qual, float, n);
-        REGROW(r->ac, int32_t, (size_t)n*M); REGROW(r->an, int32_t, n); REGROW(r->site_flags, uint32_t, n);
-        REGROW(r->gt, int32_t, 2*(size_t)n*S);
-        if ( want_gq ) REGROW(r->gq, int32_t, (size_t)n*S);
-        REGROW(s->adj_pl_off, int64_t, n);
-    }
-    if ( pl_need > s->adj_pl_cap )
-    {
-        s->adj_pl_cap = pl_need;
-        REGROW(in->pl, int32_t, pl_need); REGROW(r->pl, int32_t, pl_need);
-        if ( s->res.gp ) REGROW(r->gp, float, pl_need);
-    }
-    int64_t off = 0; int k = 0;
-    for (int i=0; i<s->n; i++)
-    {
-        if ( !(s->res.site_flags[i] & MCB_SITE_NEAR_TIE) ) continue;
-        const int64_t len = (int64_t)S*s->nals[i]*(s->nals[i]+1)/2;
-        memcpy((int32_t*)in->pl + off, s->pl + s->pl_off[i], (size_t)len*4);
-        ((int64_t*)in->pl_off)[k] = s->adj_pl_off[k] = off;
-        off += (len + 3) & ~(int64_t)3;
-        ((uint8_t*)in->nals)[k] = s->nals[i]; ((uint8_t*)in->unseen)[k] = s->unseen[i]; ((uint8_t*)in->nqs)[k] = s->nqs[i];
-        ((uint16_t*)in->ploidy_id)[k] = s->ploidy_id[i];
-        memcpy((float*)in->qs + (size_t)k*M, s->qs + (size_t)i*M, sizeof(float)*M);
-        if ( b->use_prior ) { ((int32_t*)in->prior_an)[k] = s->prior_an[i]; memcpy((int32_t*)in->prior_ac + (size_t)k*M, s->prior_ac + (size_t)i*M, 4*(size_t)M); }
-        s->adj_idx[i] = k++;
-    }
-    mcb_batch q = *in;
-    q.nsites = n; q.pl_type = 4;
-    if ( !b->use_prior ) { q.prior_an = NULL; q.prior_ac = NULL; }
-    int rc = mcb_set_option(b->ctx, "exact_phase1", 1);
-    if ( !rc ) rc = mcb_call_host(b->ctx, &q, r);
-    mcb_set_option(b->ctx, "exact_phase1", 0);
-    if ( rc ) { snprintf(err, nerr, "b200_mcall: near-tie adjudication: %s (%s)\n", mcb_strerror(rc), mcb_last_cuda_error(b->ctx)); return rc; }
-    for (int j=0; j<n; j++) r->site_flags[j] |= MCB_SITE_ADJUDICATED;
-    s->adj_n = n;
-    return 0;
-}
-
 static int run_batch(b200_batcher_t *b, b200_slabs_t *s, char *err, size_t nerr)
 {
     /* ploidy vectors this batch is the first to use */
@@ -160,8 +95,6 @@ static int run_batch(b200_batcher_t *b, b200_slabs_t *s, char *err, size_t nerr)
     if ( b->use_prior ) { in.prior_an = s->prior_an; in.prior_ac = s->prior_ac; }
     int rc = mcb_call_host(b->ctx, &in, &s->res);
     if ( rc ) snprintf(err, nerr, "b200_mcall: %s (%s)\n", mcb_strerror(rc), mcb_last_cuda_error(b->ctx));
-    s->adj_n = 0;
-    if ( !rc && !b->grouped && !b->typed ) rc = adjudicate(b, s, s->res.gq != NULL, err, nerr);
     return rc;
 }
 
@@ -221,7 +154,6 @@ static void alloc_set(b200_batcher_t *b, b200_slabs_t *s, uint32_t output_tags)
     }
     s->res.gp = (output_tags & CALL_FMT_GP) ? (float*) pinned((size_t)b->pl_cap*4) : NULL;
     s->res.pl_off_out = (int64_t*) pinned(sizeof(int64_t)*R);
-    s->adj_idx = (int*) xcalloc(R, sizeof(int));
 }
 static void free_set(b200_slabs_t *s)
 {
@@ -233,11 +165,6 @@ static void free_set(b200_slabs_t *s)
     mcb_host_free(s->res.gq); mcb_host_free(s->res.gp); mcb_host_free(s->res.pl); mcb_host_free(s->res.pl_off_out);
     mcb_host_free(s->res.gt8); mcb_host_free(s->res.gq8); mcb_host_free(s->res.pl16);
     free(s->user_in); free(s->user_out);
-    free(s->adj_idx); free(s->adj_pl_off);
-    free((void*)s->adj_in.pl); free((void*)s->adj_in.pl_off); free((void*)s->adj_in.nals); free((void*)s->adj_in.unseen); free((void*)s->adj_in.nqs);
-    free((void*)s->adj_in.ploidy_id); free((void*)s->adj_in.qs); free((void*)s->adj_in.prior_an); free((void*)s->adj_in.prior_ac);
-    free(s->adj.ret); free(s->adj.als_new); free(s->adj.als_map); free(s->adj.qual); free(s->adj.ac); free(s->adj.an); free(s->adj.site_flags);
-    free(s->adj.gt); free(s->adj.gq); free(s->adj.gp); free(s->adj.pl);
 }
 
 void b200_mcall_init(b200_call_t *call)
@@ -263,6 +190,10 @@ void b200_mcall_init(b200_call_t *call)
     p.use_prior = call->use_prior;  p.device = call->device;  p.tie_eps = call->tie_eps;
     int rc = mcb_init(&b->ctx, &p);
     if ( rc ) b200_error("b200_mcall_init: %s (%s)\n", mcb_strerror(rc), b->ctx ? mcb_last_cuda_error(b->ctx) : "");
+    /* the sites whose two best allele sets are closer than tie_eps are evaluated a second time inside each mcb_call_host, with
+       the literal sample-sequential sums of logs of the reference (DESIGN.md §5): in every mode, grouped and typed included */
+    rc = mcb_set_option(b->ctx, "adjudicate", 1);
+    if ( rc ) b200_error("b200_mcall_init: %s\n", mcb_strerror(rc));
 
     const int S = b->nsmpl, M = b->max_nals, R = b->cap;
     const int64_t gmax = (int64_t)M*(M+1)/2;
@@ -444,29 +375,6 @@ int b200_mcall_result(b200_call_t *call, int i, b200_out_t *out)
     const b200_slabs_t *s = &b->set[b->current];
     const int S = b->nsmpl, M = b->max_nals;
     memset(out, 0, sizeof *out);
-    if ( s->adj_n && s->adj_idx[i] >= 0 )       /* adjudicated near tie: the second call's result stands */
-    {
-        const int j = s->adj_idx[i];
-        const mcb_result *r = &s->adj;
-        out->ret = r->ret[j];
-        out->user = s->user_out[i];
-        out->site_flags = r->site_flags[j];
-        if ( out->ret<=0 ) return 0;
-        out->als_new = r->als_new[j];
-        out->als_map = r->als_map + (size_t)j*M;
-        out->qual = r->qual[j];
-        out->ac = r->ac + (size_t)j*M;  out->an = r->an[j];
-        const int ref_gt = (out->site_flags & MCB_SITE_REF_GT) != 0;
-        out->gts = r->gt + (size_t)j*S*2;
-        out->GQs = (r->gq && !ref_gt) ? r->gq + (size_t)j*S : NULL;
-        if ( !(out->site_flags & MCB_SITE_PL_DROPPED) )
-        {
-            out->PLs = r->pl + s->adj_pl_off[j];
-            out->nPLs = S*out->ret*(out->ret+1)/2;
-            if ( r->gp && !ref_gt ) out->GPs = r->gp + s->adj_pl_off[j];
-        }
-        return 0;
-    }
     out->ret = s->res.ret[i];
     out->user = s->user_out[i];
     out->site_flags = s->res.site_flags[i];

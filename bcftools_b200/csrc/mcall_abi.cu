@@ -76,7 +76,8 @@ struct mcb_ctx
     HostSlab slab[NSLAB];
     /* options */
     int64_t opt_tile_bytes = 0, opt_ring_bytes = 0, opt_blocks_per_sm = 0, opt_slab_bytes = 64ll<<20, opt_slab_min = 8ll<<20, opt_block = 0;     /* 0 = automatic */
-    int64_t opt_exact = 0;               /* 1: near-tie adjudication -- every site through the general kernel with the literal phase 1 (KArgs.exact_phase1) */
+    int64_t opt_exact = 0;               /* 1: every site through the literal phase 1 (KArgs.exact_phase1): the general, grouped and 6..32 allele kernels */
+    int64_t opt_adjudicate = 0;          /* 1: the sites flagged MCB_SITE_NEAR_TIE are evaluated again with the literal phase 1 inside the call */
     int64_t opt_multi = 1;               /* 3-5 allele classes: the CTA-per-site kernel of mcall_multi.cu (0: the general tiled kernel) */
     int64_t opt_mm_nst = 0;              /* its ring stages per warp (0 = automatic) */
     int64_t opt_mm_nst_c[NCLASS] = {0,0,0,0,0,0};       /* ... per allele-count class */
@@ -194,6 +195,7 @@ extern "C" int mcb_set_option(mcb_ctx *ctx, const char *key, int64_t value)
         ctx->opt_gorder = value;
     }
     else if ( !strcmp(key,"exact_phase1") )  { if ( value<0 || value>1 ) return MCB_EINVAL; ctx->opt_exact = value; }
+    else if ( !strcmp(key,"adjudicate") )    { if ( value<0 || value>1 ) return MCB_EINVAL; ctx->opt_adjudicate = value; }
     else if ( !strcmp(key,"mm_nst") )        { if ( value<0 || value>4 ) return MCB_EINVAL; ctx->opt_mm_nst = value; }
     else if ( !strncmp(key,"mm_nst_",7) && key[7]>='3' && key[7]<='5' && !key[8] ) { if ( value<0 || value>4 ) return MCB_EINVAL; ctx->opt_mm_nst_c[key[7]-'0'] = value; }
     else if ( !strcmp(key,"mm_block") )      { if ( value!=0 && value!=64 && value!=128 && value!=256 ) return MCB_EINVAL; ctx->opt_mm_block = value; }
@@ -490,6 +492,48 @@ static int ensure_class_streams(mcb_ctx *ctx)
     return MCB_OK;
 }
 
+/*  In-call adjudication (option "adjudicate"), enqueued on `st` behind every site kernel of the call (the class streams have
+ *  joined it).  A scan of site_flags lists the sites flagged MCB_SITE_NEAR_TIE per allele-count class, in the class lists of
+ *  the first evaluation, which no longer needs them; then each class is launched over its list with the literal phase 1: the
+ *  general kernel (pooled, int32 or int16 PLs), the grouped kernel, the 6..32 allele kernel.  The grids are persistent and
+ *  read the list's count on the device, so an empty list costs one short launch and the host never waits.  Every output
+ *  of a listed site is overwritten, in place (KArgs.adj_pass; compacted blocks were reserved at full size, compact_out_off).
+ *  The fallback-list counts of the first evaluation (mcb_get_fallback_counts) are left as they are.
+ *  ggrid / gper_class: the grid and the per-class scratch stride of the grouped kernel (grouped calling only).  */
+static int enqueue_adjudication(mcb_ctx *ctx, const KArgs &a1, const mcb_batch *b, int32_t *lists, int32_t *counts, int list_stride, int pl_es,
+                                KernelScratch &sc, int ggrid, size_t gper_class, cudaStream_t st, int *launches)
+{
+    CK(cudaMemsetAsync(counts, 0, sizeof(int32_t)*2*NCLASS, st));          /* class counts + work counters */
+    CK(launch_collect_near_ties(b->nals, b->nsites, a1.site_flags, lists, counts, list_stride, st));
+    KArgs a = a1;
+    a.exact_phase1 = 1; a.adj_pass = 1; a.adj_reserve = 0;
+    a.fb_list = nullptr; a.fb_count = nullptr; a.mm_sums = nullptr;
+    const bool ploidy = ctx->any_nondiploid, gpk = a.gp && (a.output_tags & MCB_CALL_FMT_GP);
+    int n = 1;
+    for (int nals=1; nals<=5; nals++, n++)
+    {
+        a.site_list = lists + (size_t)nals*list_stride; a.site_count = counts + nals;
+        a.work_counter = counts + NCLASS + nals;
+        if ( ctx->ngroups > 1 ) { CK(launch_groups_kernel(nals, a, (char*)sc.grp + (size_t)(nals-1)*gper_class, ggrid, st)); continue; }
+        size_t ring; tile_geometry(ctx, nals, pl_es, &a.tile_smpl, &a.nstage, &ring);
+        const int block = (pl_es==2 || gpk) ? 128 : class_block(ctx, nals);
+        int nb = 1;
+        CK(site_kernel_occupancy(nals, ploidy, gpk, block, pl_es, ring, &nb));
+        if ( nb<1 ) return cuda_fail(ctx, cudaErrorLaunchOutOfResources, "site kernel does not fit on an SM");
+        const int grid = (int)std::min<int64_t>((int64_t)b->nsites, (int64_t)ctx->nsm*nb);
+        cudaError_t le = launch_site_kernel(nals, ploidy, gpk, block, pl_es, a, grid, ring, st);
+        if ( le!=cudaSuccess ) return cuda_fail(ctx, le, "near-tie adjudication: site kernel");
+    }
+    if ( ctx->p.max_nals > 5 && pl_es == 4 )        /* 6..32 alleles (class 0) */
+    {
+        int rc = enqueue_class0(ctx, a, b, nullptr, lists, counts, pl_es, sc, st);
+        if ( rc ) return rc;
+        n++;
+    }
+    *launches += n;
+    return MCB_OK;
+}
+
 static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_t *lists, int32_t *counts, int list_stride, unsigned long long *cursor, KernelScratch &sc, cudaStream_t st)
 {
     CK(cudaMemsetAsync(counts, 0, sizeof(int32_t)*NCOUNTS, st));
@@ -508,7 +552,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
     a.nsmpl = ctx->p.nsmpl; a.max_nals = ctx->p.max_nals; a.flag = ctx->p.flag; a.output_tags = ctx->p.output_tags;
     a.theta = ctx->theta_log; a.tie_eps = ctx->p.tie_eps; a.use_prior = ctx->p.use_prior;
     a.exact_phase1 = (int)ctx->opt_exact;
-    if ( ctx->opt_exact && ctx->ngroups > 1 ) return MCB_EINVAL;   /* the adjudication path covers pooled calling */
+    a.adj_reserve = ctx->opt_adjudicate && r->pl_off_out;     /* flagged sites reserve their full-G compacted block (compact_out_off) */
     const bool ploidy = ctx->any_nondiploid;
     const int pl_es = b->pl_type==2 ? 2 : 4;
     if ( b->pl_type!=0 && b->pl_type!=4 && b->pl_type!=2 ) return MCB_EINVAL;
@@ -553,7 +597,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
             if ( gfork ) CK(cudaStreamWaitEvent(cs, ctx->cev_fork, 0));
             /* two alleles, up to 32 groups with ascending member lists, no FORMAT/GP: the warp-per-site kernel; what it has no
                code for comes back on a fallback list that the general grouped kernel walks */
-            if ( nals==2 && ctx->opt_bgroups && ctx->grp_sorted && biallelic_groups_ok(a.nsmpl, ctx->ngroups) && !(a.gp && (a.output_tags & MCB_CALL_FMT_GP)) )
+            if ( nals==2 && ctx->opt_bgroups && !ctx->opt_exact && ctx->grp_sorted && biallelic_groups_ok(a.nsmpl, ctx->ngroups) && !(a.gp && (a.output_tags & MCB_CALL_FMT_GP)) )
             {
                 KArgs ab = a;
                 ab.fb_list = lists + (size_t)(NCLASS + nals)*list_stride;
@@ -571,6 +615,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
             launches++;
         }
         { int rc0 = enqueue_class0(ctx, a, b, r, lists, counts, pl_es, sc, st); if ( rc0 ) return rc0; }
+        if ( ctx->opt_adjudicate ) { int rca = enqueue_adjudication(ctx, a, b, lists, counts, list_stride, pl_es, sc, grid, per_class, st, &launches); if ( rca ) return rca; }
         ctx->stats[0] += launches + 1;
         ctx->stats[1] += b->nsites;
         ctx->kev_valid = gtiming;
@@ -749,6 +794,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
     ctx->kev_valid = timing;
     { int rc0 = enqueue_class0(ctx, a, b, r, lists, counts, pl_es, sc, st); if ( rc0 ) return rc0; }
     launches++;
+    if ( ctx->opt_adjudicate ) { int rca = enqueue_adjudication(ctx, a, b, lists, counts, list_stride, pl_es, sc, 0, 0, st, &launches); if ( rca ) return rca; }
     ctx->stats[0] += launches;
     ctx->stats[1] += b->nsites;
     return MCB_OK;
@@ -757,6 +803,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
 extern "C" int mcb_call_device(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, void *cuda_stream)
 {
     if ( !ctx || !b || !r || !r->ret || b->nsites<0 || !b->pl || !b->pl_off || !b->nals ) return MCB_EINVAL;
+    if ( ctx->opt_adjudicate && !r->site_flags ) return MCB_EINVAL;     /* the flagged sites are found from site_flags */
     if ( b->nsites==0 ) return MCB_OK;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t) cuda_stream;
@@ -806,6 +853,7 @@ template<typename T> static cudaError_t launch_narrow(const int32_t *src, T *dst
 extern "C" int mcb_call_host(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r)
 {
     if ( !ctx || !b || !r || !r->ret || b->nsites<0 || !b->pl || !b->pl_off || !b->nals ) return MCB_EINVAL;
+    if ( ctx->opt_adjudicate && !r->site_flags ) return MCB_EINVAL;     /* the flagged sites are found from site_flags */
     if ( b->nsites==0 ) return MCB_OK;
     CK(cudaSetDevice(ctx->device));
     const int S = ctx->p.nsmpl, M = ctx->p.max_nals, R = b->nsites;

@@ -553,9 +553,7 @@ __global__ void __launch_bounds__(BW_MAXWARP*32, BW_MINCTA) mcall_biallelic_warp
                 long long off = site_off;
                 if ( a.pl_off_out )
                 {
-                    off = -1;
-                    if ( !pl_dropped && !ret_early )
-                        off = (long long)atomicAdd(a.pl_cursor, (unsigned long long)(((long long)S*(nals_new*(nals_new+1)/2) + 3) & ~3ll));
+                    off = compact_out_off<false>(a, site, S, 2, nals_new, !pl_dropped && !ret_early, flags);
                     a.pl_off_out[site] = off;
                 }
                 if ( pl_dropped ) flags |= MCB_SITE_PL_DROPPED;

@@ -563,9 +563,7 @@ __global__ void __launch_bounds__(BG_WARPS*32, BG_MINCTA) mcall_biallelic_groups
             long long off = site_off;
             if ( a.pl_off_out && !rec.fallback )
             {
-                off = -1;
-                if ( !rec.pl_dropped && !rec.ret_early )
-                    off = (long long)atomicAdd(a.pl_cursor, (unsigned long long)(((long long)S*(nals_new*(nals_new+1)/2) + 3) & ~3ll));
+                off = compact_out_off<false>(a, site, S, 2, nals_new, !rec.pl_dropped && !rec.ret_early, flags);
                 a.pl_off_out[site] = off;
             }
             rec.out_off = off;

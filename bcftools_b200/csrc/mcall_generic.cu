@@ -8,7 +8,8 @@
  *             missing-value fill in place (mcall.c:495-527), store the row's sum (sequential, index order) and a
  *             "has data" flag.
  *    phase A  one warp per group; the allele sets are taken 32 at a time (lane <-> set) and the group's samples are
- *             walked once per chunk of sets, every lane accumulating its set as an exponent-tracked product.
+ *             walked once per chunk of sets, every lane accumulating its set as an exponent-tracked product.  With
+ *             KArgs.exact_phase1 every lane sums log(val) sample by sample instead (the literal mcall_find_best_alleles).
  *    phase B  thread 0 combines the groups (mcall.c:1546-1577).
  *    phase C  one thread per sample: literal mcall_call_genotypes (mcall.c:745-886) on the <= 6 genotypes of the
  *             group's <= 3 selected alleles, GQ/GP, PL trimming, AC.
@@ -226,7 +227,7 @@ __global__ void __launch_bounds__(XBLOCK) mcall_generic_kernel(const KArgs a, XG
             }
             if ( lane<nals ) grec[g].q[lane] = (double)qa;
             /* ---- allele sets, 32 at a time */
-            double run_best = -CUDART_INF, run_second = -CUDART_INF, run_mx = -CUDART_INF, run_term = 0, ref_lk = 0;
+            double run_best = -CUDART_INF, run_second = -CUDART_INF, run_mx = -CUDART_INF, run_term = 0, ref_lk = 0, run_lse = -CUDART_INF;
             uint32_t run_als = 0; bool any = false;
             uint32_t wflags = 0;
             for (int c0=0; c0<nsub; c0+=32)
@@ -269,7 +270,7 @@ __global__ void __launch_bounds__(XBLOCK) mcall_generic_kernel(const KArgs a, XG
                     }
                 }
                 double M = 1, MN = 1; int E = 0, EN = 0, cnt = 0, since = 0;
-                if ( live )
+                if ( live && !a.exact_phase1 )
                     for (int i=beg; i<end; i++)
                     {
                         const int s = grouped ? a.grp_smpl[i] : i;
@@ -303,9 +304,46 @@ __global__ void __launch_bounds__(XBLOCK) mcall_generic_kernel(const KArgs a, XG
                         if ( ++since >= 256 ) { acc_renorm(M, E); acc_renorm(MN, EN); since = 0; }
                     }
                 double lk = 0;
-                const bool cand = live && cnt>0;
+                bool cand = live && cnt>0;
                 if ( cand ) lk = (log(M) + (double)(E - 1023*cnt)*LN2) - (log(MN) + (double)(EN - 1023*cnt)*LN2);
-                if ( inrange ) for (int j=0; j<nonref; j++) lk += a.theta;
+                if ( a.exact_phase1 && live )
+                {
+                    /* literal phase 1 (options exact_phase1 / adjudicate): the group's samples strictly in order, pdg = p/sum by
+                       IEEE division (set_pdg, mcall.c:451-544), val in the reference's expression order, lk += log(val)
+                       (mcall.c:601-698) -- the numerics of exact_set_lk (mcall_device.cuh) for a set of any 32 alleles */
+                    double xt = 0; bool xset = false;
+                    for (int i=beg; i<end; i++)
+                    {
+                        const int s = grouped ? a.grp_smpl[i] : i;
+                        const double sum = fsum[s];
+                        if ( sum==0 ) continue;
+                        const int *row = fpl + (size_t)s*G;
+                        auto pdg = [&](int t) -> double { return __ddiv_rn(xpl_to_p(s_pl2p, a.tab, row[tix[t]], &wflags), sum); };
+                        const int pld = ploidy[s];
+                        double val = 0;
+                        if ( single ) val = pdg(0);
+                        else if ( pld==2 )
+                        {
+                            val = __dadd_rn(__dmul_rn(cd[0], pdg(0)), __dmul_rn(cd[1], pdg(1)));
+                            if ( sc<0 ) val = __dadd_rn(val, __dmul_rn(cd[3], pdg(3)));
+                            else
+                            {
+                                val = __dadd_rn(val, __dmul_rn(cd[2], pdg(2)));
+                                val = __dadd_rn(val, __dmul_rn(cd[3], pdg(3)));
+                                val = __dadd_rn(val, __dmul_rn(cd[4], pdg(4)));
+                                val = __dadd_rn(val, __dmul_rn(cd[5], pdg(5)));
+                            }
+                        }
+                        else if ( pld==1 )
+                        {
+                            val = __dadd_rn(__dmul_rn(ch[0], pdg(0)), __dmul_rn(ch[1], pdg(1)));
+                            if ( sc>=0 ) val = __dadd_rn(val, __dmul_rn(ch[2], pdg(2)));
+                        }
+                        if ( val != 0 ) { xt = __dadd_rn(xt, log(val)); xset = true; }
+                    }
+                    cand = xset; lk = xt;
+                }
+                if ( inrange ) for (int j=0; j<nonref; j++) lk = __dadd_rn(lk, a.theta);
                 const bool in_sum = cand && !(single && sa==0);
                 if ( c0==0 ) ref_lk = __shfl_sync(0xffffffffu, lk, 0);
                 /* chunk maximum (first in enumeration order), then merge with the running state; earlier chunks win ties */
@@ -324,7 +362,8 @@ __global__ void __launch_bounds__(XBLOCK) mcall_generic_kernel(const KArgs a, XG
                     if ( !any || best > run_best ) { run_second = fmax(run_second, fmax(any ? run_best : -CUDART_INF, second)); run_best = best; run_als = cals; any = true; }
                     else run_second = fmax(run_second, best);
                 }
-                /* running log-sum-exp over the sets that enter lk_sum */
+                /* running log-sum-exp over the sets that enter lk_sum (literal path: the reference's logsumexp2 chain) */
+                if ( a.exact_phase1 ) run_lse = exact_lk_sum(lk, in_sum, 32, run_lse);
                 double mx = in_sum ? lk : -CUDART_INF;
                 for (int off=16; off; off>>=1) mx = fmax(mx, __shfl_xor_sync(0xffffffffu, mx, off));
                 if ( mx > -CUDART_INF )
@@ -345,7 +384,7 @@ __global__ void __launch_bounds__(XBLOCK) mcall_generic_kernel(const KArgs a, XG
                 for (int j=0; j<nals; j++) n += (r.als>>j)&1u;
                 r.nals = n; r.has_max = any;
                 r.ref_lk = ref_lk;
-                r.lk_sum = run_mx > -CUDART_INF ? run_mx + log(run_term) : -CUDART_INF;
+                r.lk_sum = a.exact_phase1 ? run_lse : (run_mx > -CUDART_INF ? run_mx + log(run_term) : -CUDART_INF);
                 r.qual = any ? -4.343*(r.ref_lk - logsumexp2_dev(r.lk_sum, r.ref_lk)) : -CUDART_INF;
                 uint32_t f = wflags;
                 if ( any && run_best - run_second < a.tie_eps ) f |= MCB_SITE_NEAR_TIE;
@@ -360,6 +399,7 @@ __global__ void __launch_bounds__(XBLOCK) mcall_generic_kernel(const KArgs a, XG
         if ( tid==0 )
         {
             uint32_t als_new = 0, flags = st.flags;
+            if ( a.adj_pass ) flags |= MCB_SITE_NEAR_TIE | MCB_SITE_ADJUDICATED;
             double ref_lk = -CUDART_INF, lk_sum = -CUDART_INF, max_qual = -CUDART_INF;
             for (int g=0; g<ngrp; g++)
             {
@@ -391,9 +431,7 @@ __global__ void __launch_bounds__(XBLOCK) mcall_generic_kernel(const KArgs a, XG
                 long long off = site_off;
                 if ( a.pl_off_out )
                 {
-                    off = -1;
-                    if ( !st.pl_dropped && !st.ret_early )
-                        off = (long long)atomicAdd(a.pl_cursor, (unsigned long long)(((long long)nsmpl*(nals_new*(nals_new+1)/2) + 3) & ~3ll));
+                    off = compact_out_off<true>(a, site, nsmpl, nals, nals_new, !st.pl_dropped && !st.ret_early, flags);
                     a.pl_off_out[site] = off;
                 }
                 st.out_off = off;

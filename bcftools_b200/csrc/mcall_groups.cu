@@ -5,6 +5,8 @@
  *             FORMAT/AD in float32, sequential in group order exactly like mcall.c:1478-1503 (lane a <-> allele a);
  *             then the group's samples are walked sequentially, every lane accumulating its own set as an
  *             exponent-tracked product (same numerics as the pooled kernel); the set epilogue is the pooled one.
+ *             KArgs.exact_phase1 (options exact_phase1 / adjudicate): every group takes the sample-parallel path and lane k
+ *             then walks the group's member list once more with the literal sums of logs (exact_set_lk, mcall_device.cuh).
  *    phase B  thread 0 combines the groups: als_new = OR of the groups' sets | REF, the QUAL candidate of the group
  *             with the largest QUAL (mcall.c:1546-1575), trimming maps (mcall.c:547-570).
  *    phase C  one THREAD per sample: literal mcall_call_genotypes() with the sample's own group record
@@ -162,7 +164,7 @@ __global__ void __launch_bounds__(GBLOCK, (NALS<=3 ? GMINB3 : (NALS==4 ? GMINB4 
         for (int g=warp; g<ngrp; g+=GNW)
         {
             const int beg = a.grp_off[g], end = a.grp_off[g+1];
-            if ( end-beg >= BIG_GROUP ) continue;       /* handled by the whole CTA below */
+            if ( end-beg >= BIG_GROUP || a.exact_phase1 ) continue;     /* handled below (the literal phase 1 always is) */
             /* ---- quality sums from FORMAT/AD: float32, sequential over the group's samples (mcall.c:1484-1501) */
             float qa = 0;
             if ( site_ad )
@@ -411,7 +413,7 @@ __global__ void __launch_bounds__(GBLOCK, (NALS<=3 ? GMINB3 : (NALS==4 ? GMINB4 
         for (int g=0, big_i=0; g<ngrp; g++)
         {
             const int beg = a.grp_off[g], end = a.grp_off[g+1], ng = end-beg;
-            if ( ng < BIG_GROUP ) continue;
+            if ( ng < BIG_GROUP && !a.exact_phase1 ) continue;
             if ( (big_i++ % GNW) != warp ) continue;
             {
                 /* quality sums (float32, group order), -F prior, normalisation: as in the warp path above */
@@ -730,6 +732,21 @@ __global__ void __launch_bounds__(GBLOCK, (NALS<=3 ? GMINB3 : (NALS==4 ? GMINB4 
                     for (int j=0; j<nonref; j++) lk += a.theta;
                     cand = set; in_sum = set;
                 }
+                if ( a.exact_phase1 )
+                {
+                    /* literal phase 1 (options exact_phase1 / adjudicate): lane k walks the group's member list strictly in
+                       order with the reference's pdg, val and log (mcall.c:601-698); the products above still filled ssum[] */
+                    bool is_set = false;
+                    uint32_t xflags = 0;
+                    const double xlk = exact_set_lk<NALS,true,int32_t>(site_pl, a.grp_smpl + beg, ng, unseen, ploidy, smem_u32(s_pl2p), a.tab, lane,
+                                                                       s_cfp[warp], s_cft[warp], live, a.theta, &is_set, &xflags);
+                    if ( lane < NSUB )
+                    {
+                        lk = xlk; cand = is_set;
+                        in_sum = is_set && lane != 0;
+                        if ( lane==0 && !is_set ) lk = 0;
+                    }
+                }
                 double best = cand ? lk : -CUDART_INF; int best_lane = cand ? lane : 64;
                 #pragma unroll
                 for (int off=16; off; off>>=1)
@@ -747,7 +764,8 @@ __global__ void __launch_bounds__(GBLOCK, (NALS<=3 ? GMINB3 : (NALS==4 ? GMINB4 
                 double term = in_sum ? exp(lk - mx) : 0.0;
                 #pragma unroll
                 for (int off=16; off; off>>=1) term += __shfl_xor_sync(0xffffffffu, term, off);
-                const double g_lk_sum = mx > -CUDART_INF ? mx + log(term) : -CUDART_INF;
+                double g_lk_sum = mx > -CUDART_INF ? mx + log(term) : -CUDART_INF;
+                if ( a.exact_phase1 ) g_lk_sum = exact_lk_sum(lk, in_sum, NSUB, -CUDART_INF);     /* running logsumexp2 in enumeration order */
                 const double g_ref_lk = __shfl_sync(0xffffffffu, lk, 0);
                 const uint32_t g_als = __shfl_sync(0xffffffffu, mask, best_lane & 31);
                 if ( lane==0 )
@@ -772,6 +790,7 @@ __global__ void __launch_bounds__(GBLOCK, (NALS<=3 ? GMINB3 : (NALS==4 ? GMINB4 
         if ( tid==0 )
         {
             uint32_t als_new = 0, flags = st.flags;
+            if ( a.adj_pass ) flags |= MCB_SITE_NEAR_TIE | MCB_SITE_ADJUDICATED;
             double ref_lk = -CUDART_INF, lk_sum = -CUDART_INF, max_qual = -CUDART_INF;
             for (int g=0; g<ngrp; g++)
             {
@@ -804,9 +823,7 @@ __global__ void __launch_bounds__(GBLOCK, (NALS<=3 ? GMINB3 : (NALS==4 ? GMINB4 
                 long long off = site_off;
                 if ( a.pl_off_out )
                 {
-                    off = -1;
-                    if ( !st.pl_dropped && !st.ret_early )
-                        off = (long long)atomicAdd(a.pl_cursor, (unsigned long long)(((long long)nsmpl*(nals_new*(nals_new+1)/2) + 3) & ~3ll));
+                    off = compact_out_off<true>(a, site, nsmpl, NALS, nals_new, !st.pl_dropped && !st.ret_early, flags);
                     a.pl_off_out[site] = off;
                 }
                 st.out_off = off;

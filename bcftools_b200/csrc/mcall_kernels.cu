@@ -159,108 +159,6 @@ __device__ __forceinline__ bool load_sample_w(uint32_t row_s, uint32_t pl2p_s, b
 }
 
 /* ------------------------------------------------------------------------------------------------
- *  Near-tie adjudication (KArgs.exact_phase1): the LITERAL mcall_find_best_alleles (mcall.c:591-710) for one allele
- *  set per lane of warp 0 -- every sample's pdg = p/sum by IEEE division (set_pdg, mcall.c:451-544), val in the
- *  reference's expression order, lk_tot += log(val) strictly in sample order -- instead of the exponent-tracked
- *  products.  Two orders of magnitude slower (the whole warp walks the site sample by sample and takes one log() per
- *  sample and set), so it only runs on request: the host batcher re-submits the sites that came back with
- *  MCB_SITE_NEAR_TIE.  What still separates it from the reference is the last bit of log() itself (libdevice vs glibc).
- *  lane < NALS: {lane}; then pairs, then triples, in enumeration order.  cf5 / cf9: the set's coefficients as laid out
- *  by the set-up above.  Returns lk_tot (theta included); *is_set = lk_tot_set.
- * ---------------------------------------------------------------------------------------------- */
-template<int NALS, bool PLOIDY, typename PT>
-static __device__ __noinline__ double exact_set_lk(const PT *site_pl, int nsmpl, int unseen, const uint8_t *ploidy, uint32_t pl2p_s,
-                                                   const DevTables *tab, int lane, const double *cf_pair, const double *cf_tri,
-                                                   uint32_t live, double theta, bool *is_set, uint32_t *flags)
-{
-    using S = Shape<NALS>;
-    constexpr int G = S::G, NPAIR = S::NPAIR, NSUB = S::NSUB;
-    int sa = 0, sb = -1, sc = -1;
-    bool lv = lane < NALS;
-    const double *cf = nullptr;
-    if ( lane < NALS ) sa = lane;
-    else if ( lane < NALS+NPAIR )
-    {
-        const int k = lane-NALS; sa = 1; while ( sa*(sa+1)/2 <= k ) sa++;
-        sb = k - sa*(sa-1)/2; cf = cf_pair + k*5; lv = (live >> k) & 1u;
-    }
-    else if ( lane < NSUB )
-    {
-        const int k = lane-NALS-NPAIR; sa = 2; while ( (sa+1)*sa*(sa-1)/6 <= k ) sa++;
-        const int r = k - sa*(sa-1)*(sa-2)/6; sb = 1; while ( sb*(sb+1)/2 <= r ) sb++;
-        sc = r - sb*(sb-1)/2; cf = cf_tri + k*9; lv = (live >> (NPAIR+k)) & 1u;
-    }
-    double lk_tot = 0; bool lk_set = false;
-    #pragma unroll 1
-    for (int s=0; s<nsmpl; s++)
-    {
-        /* set_pdg for this sample (every lane the same row: broadcast loads) */
-        int pl[G]; int orv = 0;
-        for (int j=0; j<G; j++) { pl[j] = PLType<PT>::widen((int)site_pl[(size_t)s*G + j]); orv |= pl[j]; }
-        bool data = orv != 0;
-        if ( orv < 0 )
-        {
-            int j;
-            data = true;
-            for (j=0; j<G; j++) { if ( pl[j]==I32_VEC_END ) { data = false; break; } if ( pl[j]==I32_MISSING ) break; }
-            if ( data && (j==0 || j==G) ) data = false;
-            if ( data )
-            {
-                j = 0;
-                for (int ia=0; ia<NALS && data; ia++)
-                    for (int ib=0; ib<=ia; ib++, j++)
-                    {
-                        if ( pl[j]==I32_MISSING )
-                        {
-                            int k = gt_idx(ia,unseen);
-                            if ( pl[k]==I32_MISSING ) k = gt_idx(ib,unseen);
-                            if ( pl[k]==I32_MISSING ) k = gt_idx(unseen,unseen);
-                            pl[j] = pl[k]==I32_MISSING ? 255 : pl[k];
-                        }
-                        else if ( pl[j] < 0 ) { data = false; break; }
-                    }
-            }
-            if ( data ) { orv = 0; for (int j2=0; j2<G; j2++) orv |= pl[j2]; data = orv > 0; }
-        }
-        if ( !data ) continue;                  /* pdg = 0 everywhere: neither log(*pdg) nor log(val) is taken */
-        double pdg[G], sum = 0;
-        for (int j=0; j<G; j++)
-        {
-            pdg[j] = (unsigned)pl[j] < 256u ? lds64(pl2p_s + 8u*(uint32_t)pl[j]) : big_pl_to_p(tab, pl[j], flags);
-            sum = j ? __dadd_rn(sum, pdg[j]) : pdg[j];
-        }
-        for (int j=0; j<G; j++) pdg[j] = __ddiv_rn(pdg[j], sum);
-        const int pld = PLOIDY ? (int)ploidy[s] : 2;
-        double val = 0;
-        if ( sb < 0 ) val = pdg[hom_idx(sa)];                                   /* mcall.c:607-611: every sample, whatever its ploidy */
-        else if ( !lv ) continue;
-        else if ( sc < 0 )
-        {
-            if ( pld==2 ) val = __dadd_rn(__dadd_rn(__dmul_rn(cf[0], pdg[hom_idx(sa)]), __dmul_rn(cf[1], pdg[hom_idx(sb)])), __dmul_rn(cf[2], pdg[gt_idx(sa,sb)]));
-            else if ( pld==1 ) val = __dadd_rn(__dmul_rn(cf[3], pdg[hom_idx(sa)]), __dmul_rn(cf[4], pdg[hom_idx(sb)]));
-        }
-        else
-        {
-            if ( pld==2 )
-                val = __dadd_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dadd_rn(__dmul_rn(cf[0], pdg[hom_idx(sa)]), __dmul_rn(cf[1], pdg[hom_idx(sb)])),
-                      __dmul_rn(cf[2], pdg[hom_idx(sc)])), __dmul_rn(cf[3], pdg[gt_idx(sa,sb)])), __dmul_rn(cf[4], pdg[gt_idx(sa,sc)])), __dmul_rn(cf[5], pdg[gt_idx(sb,sc)]));
-            else if ( pld==1 )
-                val = __dadd_rn(__dadd_rn(__dmul_rn(cf[6], pdg[hom_idx(sa)]), __dmul_rn(cf[7], pdg[hom_idx(sb)])), __dmul_rn(cf[8], pdg[hom_idx(sc)]));
-        }
-        if ( val != 0 ) { lk_tot = __dadd_rn(lk_tot, site_log(val)); lk_set = true; }
-    }
-    if ( sb < 0 ) { if ( sa > 0 ) lk_tot = __dadd_rn(lk_tot, theta); }
-    else
-    {
-        if ( sa != 0 ) lk_tot = __dadd_rn(lk_tot, theta);
-        if ( sb != 0 ) lk_tot = __dadd_rn(lk_tot, theta);
-        if ( sc > 0 ) lk_tot = __dadd_rn(lk_tot, theta);
-    }
-    *is_set = lk_set && (sb < 0 || lv) && lane < NSUB;
-    return lk_tot;
-}
-
-/* ------------------------------------------------------------------------------------------------
  *  the fused kernel
  * ---------------------------------------------------------------------------------------------- */
 template<int NALS, int BLOCK> struct MinBlocks
@@ -690,7 +588,7 @@ __global__ void __launch_bounds__(BLOCK, (MinBlocks<NALS,BLOCK>::value)) mcall_s
             {
                 bool is_set = false;
                 uint32_t xflags = 0;
-                const double xlk = exact_set_lk<NALS,PLOIDY,PT>(site_pl, nsmpl, unseen, ploidy, pl2p_s, a.tab, lane, sh.cf_pair, sh.cf_tri, live, a.theta, &is_set, &xflags);
+                const double xlk = exact_set_lk<NALS,PLOIDY,PT>(site_pl, nullptr, nsmpl, unseen, ploidy, pl2p_s, a.tab, lane, sh.cf_pair, sh.cf_tri, live, a.theta, &is_set, &xflags);
                 if ( lane < NSUB )
                 {
                     lk = xlk; cand = is_set;
@@ -719,17 +617,7 @@ __global__ void __launch_bounds__(BLOCK, (MinBlocks<NALS,BLOCK>::value)) mcall_s
             for (int off=16; off; off>>=1) term += __shfl_xor_sync(0xffffffffu, term, off);
             double grp_lk_sum = mx > -CUDART_INF ? mx + site_log(term) : -CUDART_INF;
             if ( a.exact_phase1 )       /* ... and lk_sum as the reference's running logsumexp2 in enumeration order (mcall.c:573-585) */
-            {
-                double run = -CUDART_INF;
-                #pragma unroll 1
-                for (int k=0; k<NSUB; k++)
-                {
-                    const double v = __shfl_sync(0xffffffffu, lk, k);
-                    const int f = __shfl_sync(0xffffffffu, (int)in_sum, k);
-                    if ( f ) run = v > run ? site_log(1 + site_exp(run - v)) + v : site_log(1 + site_exp(v - run)) + run;
-                }
-                grp_lk_sum = run;
-            }
+                grp_lk_sum = exact_lk_sum(lk, in_sum, NSUB, -CUDART_INF);
             const double grp_ref_lk = __shfl_sync(0xffffffffu, lk, 0);
             const uint32_t grp_als = __shfl_sync(0xffffffffu, mask, best_lane & 31);
 
@@ -746,6 +634,7 @@ __global__ void __launch_bounds__(BLOCK, (MinBlocks<NALS,BLOCK>::value)) mcall_s
                 }
                 double gap = any ? best - second : CUDART_INF;
                 if ( any && gap < a.tie_eps ) flags |= MCB_SITE_NEAR_TIE;
+                if ( a.adj_pass ) flags |= MCB_SITE_NEAR_TIE | MCB_SITE_ADJUDICATED;
                 uint32_t als_new = gals | 1u;               /* mcall.c:1552, 1564 */
                 int is_variant = als_new!=1;
                 int ret_early = ((a.flag & MCB_CALL_VARONLY) && !is_variant) || (flags & MCB_SITE_NO_QS);
@@ -773,9 +662,7 @@ __global__ void __launch_bounds__(BLOCK, (MinBlocks<NALS,BLOCK>::value)) mcall_s
                     long long off = site_off;
                     if ( a.pl_off_out )
                     {
-                        off = -1;
-                        if ( !sh.pl_dropped && !ret_early )
-                            off = (long long)atomicAdd(a.pl_cursor, (unsigned long long)(((long long)nsmpl*(nals_new*(nals_new+1)/2) + 3) & ~3ll));
+                        off = compact_out_off<true>(a, site, nsmpl, NALS, nals_new, !sh.pl_dropped && !ret_early, flags);
                         a.pl_off_out[site] = off;
                     }
                     sh.out_off = off;
@@ -1355,6 +1242,19 @@ __global__ void classify_sites_kernel(const uint8_t *nals, int nsites, int32_t *
     lists[(size_t)cls*list_stride + pos] = i;
 }
 
+/*  In-call adjudication: the sites the first evaluation flagged MCB_SITE_NEAR_TIE, one list per allele-count class (the
+ *  layout of classify_sites_kernel).  Runs after every site kernel of the call; the hot kernels append to no list.  */
+__global__ void collect_near_ties_kernel(const uint8_t *nals, int nsites, const uint32_t *site_flags, int32_t *lists, int32_t *counts, int list_stride)
+{
+    for (int i = blockIdx.x*blockDim.x + threadIdx.x; i < nsites; i += gridDim.x*blockDim.x)
+    {
+        if ( !(site_flags[i] & MCB_SITE_NEAR_TIE) ) continue;
+        const int n = nals[i], cls = (n>=1 && n<=5) ? n : 0;
+        const int pos = atomicAdd(&counts[cls], 1);
+        lists[(size_t)cls*list_stride + pos] = i;
+    }
+}
+
 /*  sites the templated kernels do not cover (n_allele 0 or >5): reported as skipped for now  */
 __global__ void unsupported_sites_kernel(const int32_t *list, const int32_t *count, int32_t *ret, uint32_t *site_flags, const uint8_t *nals, int64_t *pl_off_out)
 {
@@ -1437,6 +1337,12 @@ cudaError_t launch_classify(const uint8_t *nals, int nsites, int32_t *lists, int
 {
     if ( nsites<=0 ) return cudaSuccess;
     classify_sites_kernel<<<(nsites+255)/256, 256, 0, st>>>(nals, nsites, lists, counts, list_stride, max_nals, ret, site_flags, pl_off_out);
+    return cudaGetLastError();
+}
+cudaError_t launch_collect_near_ties(const uint8_t *nals, int nsites, const uint32_t *site_flags, int32_t *lists, int32_t *counts, int list_stride, cudaStream_t st)
+{
+    if ( nsites<=0 ) return cudaSuccess;
+    collect_near_ties_kernel<<<(nsites+255)/256 < 1024 ? (nsites+255)/256 : 1024, 256, 0, st>>>(nals, nsites, site_flags, lists, counts, list_stride);
     return cudaGetLastError();
 }
 cudaError_t launch_unsupported(const int32_t *list, const int32_t *count, int32_t *ret, uint32_t *site_flags, const uint8_t *nals, int64_t *pl_off_out, cudaStream_t st)

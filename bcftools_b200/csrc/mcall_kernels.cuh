@@ -65,7 +65,9 @@ struct KArgs
     double theta, tie_eps;
     int use_prior;
     int tile_smpl, nstage;
-    int exact_phase1;                                           /* near-tie adjudication: literal sample-sequential sums of logs in the general kernel */
+    int exact_phase1;                                           /* literal sample-sequential sums of logs (general, grouped and 6..32 allele kernels) */
+    int adj_reserve;                                            /* compacted output: a site flagged MCB_SITE_NEAR_TIE reserves its full-G block */
+    int adj_pass;                                               /* second evaluation of the flagged sites: writes into that block in place */
 };
 
 }   // namespace mcb
@@ -74,6 +76,7 @@ namespace mcb {
 /*  launchers implemented in mcall_kernels.cu  */
 cudaError_t launch_site_kernel(int nals, bool ploidy, bool gp, int block, int pl_es, const KArgs &a, int grid, size_t ring_bytes, cudaStream_t st);
 cudaError_t launch_classify(const uint8_t *nals, int nsites, int32_t *lists, int32_t *counts, int list_stride, int max_nals, int32_t *ret, uint32_t *site_flags, int64_t *pl_off_out, cudaStream_t st);
+cudaError_t launch_collect_near_ties(const uint8_t *nals, int nsites, const uint32_t *site_flags, int32_t *lists, int32_t *counts, int list_stride, cudaStream_t st);
 cudaError_t launch_unsupported(const int32_t *list, const int32_t *count, int32_t *ret, uint32_t *site_flags, const uint8_t *nals, int64_t *pl_off_out, cudaStream_t st);
 cudaError_t site_kernel_occupancy(int nals, bool ploidy, bool gp, int block, int pl_es, size_t ring_bytes, int *blocks_per_sm);
 size_t groups_scratch_bytes(int grid, int ngroups, int nsmpl);

@@ -461,7 +461,7 @@ static __device__ __noinline__ bool mm_decide(Rec *shp, const MMSetup<NALS> *su,
         {
             a.ret[site] = 0;
             if ( a.site_flags ) a.site_flags[site] = flags;
-            if ( a.pl_off_out ) a.pl_off_out[site] = -1;
+            if ( a.pl_off_out ) a.pl_off_out[site] = compact_out_off<false>(a, site, nsmpl, NALS, nals_new, false, flags);
             sh.path = 0;
         }
         else
@@ -469,9 +469,7 @@ static __device__ __noinline__ bool mm_decide(Rec *shp, const MMSetup<NALS> *su,
             long long off = su->pl_off;
             if ( a.pl_off_out )
             {
-                off = -1;
-                if ( !pl_dropped )
-                    off = (long long)atomicAdd(a.pl_cursor, (unsigned long long)(((long long)nsmpl*(nals_new*(nals_new+1)/2) + 3) & ~3ll));
+                off = compact_out_off<false>(a, site, nsmpl, NALS, nals_new, !pl_dropped, flags);
                 a.pl_off_out[site] = off;
             }
             if ( pl_dropped ) flags |= MCB_SITE_PL_DROPPED;

@@ -21,7 +21,7 @@ extern "C" {
 #define CALL_VARONLY   (1<<1)
 #define CALL_FMT_GQ    (1<<6)
 #define CALL_FMT_GP    (1<<7)
-#define B200_SITE_ADJUDICATED (1u<<9)   /* b200_out_t.site_flags: the record's near tie was re-evaluated in the reference's summation order */
+#define B200_SITE_ADJUDICATED MCB_SITE_ADJUDICATED   /* b200_out_t.site_flags: the record's near tie was re-evaluated in the reference's summation order */
 
 typedef struct b200_batcher b200_batcher_t;
 
@@ -43,12 +43,14 @@ typedef struct
     int      device;            /* CUDA device ordinal */
     int      bcf_typed;         /* 1: BCF typed vectors both ways (SURVEY.md 8f N1): FORMAT/PL is handed over as the record's own
                                    int8/int16 vector (b200_rec_t.PL_typed, e.g. bcf_fmt_t.p or b200_bcf_fmt_t.p) and GT / GQ / PL
-                                   come back as int8 / int8 / int16 vectors (b200_out_t.gts8 / GQs8 / PLs16); pooled calling only */
+                                   come back as int8 / int8 / int16 vectors (b200_out_t.gts8 / GQs8 / PLs16); pooled calling only.
+                                   Near ties are adjudicated on the device from the int16 PLs as in the int32 mode */
     int      async_flush;       /* 1: a full batch is handed to the GPU in the background and b200_mcall keeps queuing into the second
                                    slab set; the results it then reports are those of the PREVIOUS batch (see b200_mcall_flush_async) */
     double   tie_eps;           /* allele sets closer than this in log-likelihood are near ties (0 = 1e-6): such records are called a second
-                                   time with the literal sample-sequential sums of logs (mcall.c:607-611, 635-645, 680-690) and come back
-                                   with MCB_SITE_NEAR_TIE | B200_SITE_ADJUDICATED in site_flags (pooled calling, int32 PLs) */
+                                   time with the literal sample-sequential sums of logs (mcall.c:607-611, 635-645, 680-690), inside the same device
+                                   call (mcb_set_option "adjudicate"), and come back with MCB_SITE_NEAR_TIE | B200_SITE_ADJUDICATED in
+                                   site_flags.  Every mode: pooled or grouped (-G), int32 or typed PLs, 1..32 alleles */
     /* ---- owned by this layer ---- */
     b200_batcher_t *batcher;
 }

@@ -65,6 +65,8 @@ extern "C" {
 #define MCB_SITE_BAD_PRIOR     (1u<<7)   /* -F: AN < sum(AC); the reference error()s out (mcall.c:1523) */
 #define MCB_SITE_UNSUPPORTED   (1u<<8)   /* site shape not covered by the device kernels (n_allele==0, n_allele > max_nals, > 5 alleles with int16 PLs) */
 #define MCB_SITE_REF_GT       (1u<<5)   /* genotypes come from mcall_set_ref_genotypes (mcall.c:1582,1587): no GQ/GP written */
+#define MCB_SITE_ADJUDICATED  (1u<<9)   /* near tie evaluated a second time with the literal phase 1 (option "adjudicate"); always
+                                           set together with MCB_SITE_NEAR_TIE */
 
 typedef struct mcb_ctx mcb_ctx;     /* opaque; one per GPU, used from one host thread (like call_t).  Calls on one context
                                        must be stream-ordered: mcb_call_device shares work lists and scratch between calls,
@@ -139,7 +141,9 @@ typedef struct mcb_result
     int32_t  *pl;           /* trimmed FORMAT/PL, site i at pl + pl_off[i], [nsmpl][G'_i], G'_i from ret[i] */
     int64_t  *pl_off_out;   /* [nsites] optional.  If non-NULL the trimmed PLs (and GP) are written COMPACTED: site i lies
                                at pl + pl_off_out[i] (16-byte aligned blocks in no particular order, -1 when the site has
-                               no PL); the used prefix of pl is all that travels device->host in mcb_call_host */
+                               no PL); the used prefix of pl is all that travels device->host in mcb_call_host.  It never
+                               exceeds sum_i (nsmpl*G_i + 3) & ~3 int32 units, which is at most the extent of the input
+                               layout, so a buffer sized for pl_off[] indexing always suffices (also with "adjudicate") */
     /* BCF typed-vector outputs (mcb_call_host only; SURVEY.md §8f N1).  When non-NULL they are filled INSTEAD of gt / gq / pl:
        the per-sample results are narrowed on the device to the types a BCF record stores them in (what bcf_update_genotypes /
        bcf_update_format_int32 + vcf_write would re-encode the int32 arrays to), so 9 instead of 24 bytes per biallelic call
@@ -182,7 +186,13 @@ int   mcb_get_pl2p(const mcb_ctx *ctx, double *pl2p256);   /* call->pl2p (mcall.
 /*  kernel launch statistics of the last mcb_call_* (bench.py's gpu_launches / roofline):
  *  stats[0]=kernel launches, [1]=sites, [2]=algorithmic bytes read, [3]=algorithmic bytes written */
 int   mcb_get_stats(const mcb_ctx *ctx, int64_t stats[4]);
-/*  tuning knob for experiments (threads per block, tile samples, ...): see DESIGN.md */
+/*  tuning knob for experiments (threads per block, tile samples, ...): see DESIGN.md.
+ *  "adjudicate" (0|1, default 0): every site of an mcb_call_device / mcb_call_host call that comes back with MCB_SITE_NEAR_TIE
+ *  is evaluated a second time inside the same call, on the same stream and without a host synchronisation, with the literal
+ *  sample-sequential sums of logs of mcall_find_best_alleles (mcall.c:591-710).  All of the site's outputs are overwritten
+ *  by that evaluation and it carries MCB_SITE_NEAR_TIE | MCB_SITE_ADJUDICATED.  Needs result.site_flags: a call without it
+ *  returns MCB_EINVAL.  Compacted PL output (pl_off_out) stays within the documented capacity: a flagged site reserves the
+ *  block of its full genotype count.  "exact_phase1" (0|1): every site through the literal phase 1.  */
 int   mcb_set_option(mcb_ctx *ctx, const char *key, int64_t value);
 int   mcb_version(void);
 /*  device milliseconds of the site kernel per allele-count class (ms[1..5], ms[0]=sum) of the last
