@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "lib", "libmcall_b200.so")
-SOURCES = ["mcall_kernels.cu", "mcall_groups.cu", "mcall_biallelic.cu", "mcall_biallelic_groups.cu", "mcall_multi.cu", "mcall_triallelic.cu", "mcall_generic.cu", "mcall_abi.cu", "mcall_job.cu", os.path.join("host", "b200_call.c"), os.path.join("host", "b200_bcf.c"), os.path.join("host", "b200_driver.c"), os.path.join("host", "b200_vcf.c"), os.path.join("host", "b200_vcfcall.c"), os.path.join("host", "b200_pv4.c"), os.path.join("host", "b200_bcfio.c")]
+SOURCES = ["mcall_kernels.cu", "mcall_groups.cu", "mcall_biallelic.cu", "mcall_biallelic_groups.cu", "mcall_multi.cu", "mcall_triallelic.cu", "mcall_multi_warp.cu", "mcall_generic.cu", "mcall_abi.cu", "mcall_job.cu", os.path.join("host", "b200_call.c"), os.path.join("host", "b200_bcf.c"), os.path.join("host", "b200_driver.c"), os.path.join("host", "b200_vcf.c"), os.path.join("host", "b200_vcfcall.c"), os.path.join("host", "b200_pv4.c"), os.path.join("host", "b200_bcfio.c")]
 HEADERS = ["mcall_kernels.cuh", "mcall_device.cuh", "mcall_multi.cuh", os.path.join(ROOT, "include", "mcall_b200.h"), os.path.join(ROOT, "include", "b200_call.h"), os.path.join(ROOT, "include", "mcall_job.h"), os.path.join(ROOT, "include", "b200_bcf.h"), os.path.join(ROOT, "include", "b200_driver.h"), os.path.join(ROOT, "include", "b200_vcf.h"), os.path.join(ROOT, "include", "b200_vcfcall.h"), os.path.join(ROOT, "include", "b200_bcfio.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--fmad=false",   # no FMA contraction: the reference's x86-64 -O2 build has none

@@ -23,6 +23,7 @@ using namespace mcb;
 /*  one allocation per batch/slab: NCLASS class lists, NCLASS fallback lists (sites the multi-allelic kernel hands to the general one)  */
 static inline size_t lists_bytes(int cap) { return sizeof(int32_t)*(size_t)(2*NCLASS)*cap; }
 #define MAX_STAGE 16
+#define MW_L2_SHARE 0.34        /* the 4-allele warp kernel: its grid's tails of the packed copies may take this share of L2 */
 
 /*  Scratch of the grouped (-G) and generic (6..32 allele) kernels, indexed by blockIdx inside a launch.  One set per host
  *  slab and one for the device path: slabs run on independent streams, so their launches may overlap and must not share it.  */
@@ -31,11 +32,12 @@ struct KernelScratch
     void *grp = nullptr;  size_t grp_bytes = 0;
     void *gen_grp = nullptr, *gen_pl = nullptr, *gen_sum = nullptr;  int gen_grid = 0;
     double *mm_sums[6] = {};  size_t mm_sums_bytes[6] = {};     /* mcall_multi.cu: per-CTA rows of normalisers, one buffer per allele-count class (the classes run concurrently) */
+    uint8_t *mw_tail[6] = {};  size_t mw_tail_bytes[6] = {};    /* mcall_multi_warp.cu: per-warp tails of the packed copies (4-allele class) */
 };
 static void free_scratch(KernelScratch &k)
 {
     cudaFree(k.grp); cudaFree(k.gen_grp); cudaFree(k.gen_pl); cudaFree(k.gen_sum);
-    for (int i=0; i<6; i++) cudaFree(k.mm_sums[i]);
+    for (int i=0; i<6; i++) { cudaFree(k.mm_sums[i]); cudaFree(k.mw_tail[i]); }
     k = KernelScratch();
 }
 
@@ -59,7 +61,7 @@ struct HostSlab                 /* one stage of the host-path ring (H2D of slab 
 struct mcb_ctx
 {
     mcb_params p;
-    int device = 0, nsm = 0;  size_t smem_per_sm = 0;
+    int device = 0, nsm = 0;  size_t smem_per_sm = 0, l2_bytes = 0;
     double theta_log = 0;
     double pl2p[256];
     DevTables *d_tab = nullptr;
@@ -85,6 +87,7 @@ struct mcb_ctx
     int64_t opt_mm_block_c[NCLASS] = {0,0,0,0,0,0};     /* ... per allele-count class */
     int64_t opt_warp2 = -1;              /* biallelic warp-per-site kernel: -1 automatic, 0 off, n = force n warps per CTA */
     int64_t opt_warp3 = -1;              /* 3-allele warp-per-site kernel: -1 automatic, 0 off, n = at most n warps per CTA */
+    int64_t opt_warp4 = -1;              /* the same for the 4-allele warp-per-site kernel */
     int64_t opt_order = 54321;           /* launch order of the allele-count classes */
     int64_t opt_time_kernels = 0, opt_concurrent = 1;    /* class kernels on their own streams: a class fills the tail of the previous one (-3.5 % per C3 step) */
     int64_t opt_ring_bytes_c[NCLASS] = {0,0,0,0,0,0};   /* per allele-count class override of ring_bytes (0 = opt_ring_bytes) */
@@ -202,6 +205,7 @@ extern "C" int mcb_set_option(mcb_ctx *ctx, const char *key, int64_t value)
     else if ( !strncmp(key,"mm_block_",9) && key[9]>='3' && key[9]<='5' && !key[10] ) { if ( value!=0 && value!=64 && value!=128 && value!=256 ) return MCB_EINVAL; ctx->opt_mm_block_c[key[9]-'0'] = value; }
     else if ( !strcmp(key,"warp2") )         { if ( value<-1 || value>biallelic_max_warps() ) return MCB_EINVAL; ctx->opt_warp2 = value; }
     else if ( !strcmp(key,"warp3") )         { if ( value<-1 || value>triallelic_max_warps() ) return MCB_EINVAL; ctx->opt_warp3 = value; }
+    else if ( !strcmp(key,"warp4") )         { if ( value<-1 || value>multi_warp_max_warps() ) return MCB_EINVAL; ctx->opt_warp4 = value; }
     else if ( !strncmp(key,"ring_bytes_",11) && key[11]>='1' && key[11]<='5' && !key[12] ) ctx->opt_ring_bytes_c[key[11]-'0'] = value;
     else if ( !strncmp(key,"block_",6) && key[6]>='1' && key[6]<='5' && !key[7] )
     {
@@ -252,6 +256,7 @@ extern "C" int mcb_init(mcb_ctx **out, const mcb_params *params)
     CK(cudaGetDeviceProperties(&prop, ctx->device));
     ctx->nsm = prop.multiProcessorCount;
     ctx->smem_per_sm = prop.sharedMemPerMultiprocessor;
+    ctx->l2_bytes = prop.l2CacheSize;
     ctx->theta_log = init_theta(params->theta, params->init_ploidy, params->nsmpl);
 
     DevTables *t = new DevTables();
@@ -691,13 +696,27 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
         int grid = (int)std::min<int64_t>((int64_t)b->nsites, (int64_t)ctx->nsm*nb);
         cudaStream_t cs = fork ? ctx->cstream[nals] : st;
         if ( fork ) CK(cudaStreamWaitEvent(cs, ctx->cev_fork, 0));
-        /*  3-5 alleles, int32 PLs, every sample diploid, GT + GQ + PL requested: the CTA-per-site kernel of mcall_multi.cu, or for
-         *  3 alleles the warp-per-site kernel of mcall_triallelic.cu.  Sites they have no straight-line code for come back on a
-         *  fallback list, which the general kernel below walks.  */
+        /*  3-5 alleles, int32 PLs, every sample diploid, GT + GQ + PL requested: the CTA-per-site kernel of mcall_multi.cu, or the
+         *  warp-per-site kernels of mcall_triallelic.cu (3 alleles) and mcall_multi_warp.cu (4 alleles).  Sites they have no
+         *  straight-line code for come back on a fallback list, which the general kernel below walks.  */
         const bool multi_ok = nals>=3 && ctx->opt_multi && !ctx->opt_exact && !ctx->opt_block && !ctx->opt_block_c[nals] && pl_es==4 && !ploidy && !gpk && a.gt && a.gq && a.out_pl && !(a.flag & MCB_CALL_KEEPALT)
              && (a.output_tags & (MCB_CALL_FMT_GQ|MCB_CALL_FMT_GP))
              && !((reinterpret_cast<uintptr_t>(a.gt) | reinterpret_cast<uintptr_t>(a.gq) | reinterpret_cast<uintptr_t>(a.out_pl)) & 15);
-        int tw_warps = 0;
+        int tw_warps = 0, mw_warps = 0, mw_head = 0;
+        const int64_t opt_mw = ctx->opt_warp4;
+        if ( multi_ok && nals==4 && opt_mw!=0 && multi_block_for(a.nsmpl) )
+        {
+            /* as many warps as the registers allow; the packed copy that does not fit their shares of shared memory goes to an
+               L2-resident tail, which the whole grid must keep within MW_L2_SHARE of L2 (above it the CTA kernel wins) */
+            const int ncta = multi_warp_ctas_per_sm();
+            const size_t per_cta = (size_t)(ctx->smem_per_sm/ncta) - 1024;
+            int w = multi_warp_max_warps();
+            if ( opt_mw>0 ) w = std::min<int>(w, (int)opt_mw);
+            const int head = multi_warp_head(a.nsmpl, w, per_cta);
+            const double tail_all = (double)ctx->nsm*ncta*w*(double)multi_warp_tail_bytes(a.nsmpl, head);
+            const bool cta_forced = ctx->opt_mm_block || ctx->opt_mm_block_c[nals] || ctx->opt_mm_nst || ctx->opt_mm_nst_c[nals];
+            if ( head>0 && (opt_mw>0 || (!cta_forced && tail_all <= MW_L2_SHARE*(double)ctx->l2_bytes)) ) { mw_warps = w; mw_head = head; }
+        }
         if ( multi_ok && nals==3 && ctx->opt_warp3!=0 && multi_block_for(a.nsmpl) )
         {
             const int ncta = triallelic_ctas_per_sm();
@@ -721,6 +740,36 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
             {
                 char what[160];
                 snprintf(what, sizeof what, "3-allele warp kernel warps=%d grid=%d smem=%zu", tw_warps, tgrid, triallelic_smem_bytes(a.nsmpl, tw_warps));
+                return cuda_fail(ctx, le, what);
+            }
+            launches++;
+            /* the general kernel now walks the fallback list only */
+            a.site_list = am.fb_list; a.site_count = am.fb_count;
+            a.work_counter = counts + NCLASS + 16 + nals;
+            grid = std::min(grid, ctx->nsm);
+        }
+        else if ( mw_warps )
+        {
+            const int ncta = multi_warp_ctas_per_sm();
+            const int mgrid = (int)std::min<int64_t>(((int64_t)b->nsites + mw_warps - 1)/mw_warps, (int64_t)ctx->nsm*ncta);
+            const size_t tail = multi_warp_tail_bytes(a.nsmpl, mw_head);
+            if ( tail && (size_t)ctx->nsm*ncta*mw_warps*tail > sc.mw_tail_bytes[nals] )
+            {
+                CK(cudaStreamSynchronize(cs));
+                if ( sc.mw_tail[nals] ) CK(cudaFree(sc.mw_tail[nals]));
+                const size_t want = (size_t)ctx->nsm*ncta*mw_warps*tail;      /* full grid: no regrowth with the next, larger batch */
+                CK(cudaMalloc(&sc.mw_tail[nals], want));
+                sc.mw_tail_bytes[nals] = want;
+            }
+            KArgs am = a;
+            am.fb_list = lists + (size_t)(NCLASS + nals)*list_stride;
+            am.fb_count = counts + NCLASS + 8 + nals;
+            cudaError_t le = launch_multi_warp_kernel(am, mgrid, mw_warps, mw_head, sc.mw_tail[nals], cs);
+            if ( le==cudaSuccess && getenv("MCB_DEBUG_SYNC") ) le = cudaStreamSynchronize(cs);
+            if ( le!=cudaSuccess )
+            {
+                char what[160];
+                snprintf(what, sizeof what, "4-allele warp kernel warps=%d grid=%d head=%d smem=%zu", mw_warps, mgrid, mw_head, multi_warp_smem_bytes(mw_head, mw_warps));
                 return cuda_fail(ctx, le, what);
             }
             launches++;

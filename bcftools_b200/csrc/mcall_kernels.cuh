@@ -99,6 +99,14 @@ size_t triallelic_smem_bytes(int nsmpl, int nwarp);
 int triallelic_max_warps();
 int triallelic_ctas_per_sm();
 cudaError_t launch_triallelic_warp_kernel(const KArgs &a, int grid, int nwarp, cudaStream_t st);
+/*  warp-per-site kernel of the 4-allele class: the first `head` samples of the packed copy in shared memory, the rest in a
+ *  per-warp row of L2-resident global scratch (mcall_multi_warp.cu)  */
+size_t multi_warp_smem_bytes(int head, int nwarp);
+int multi_warp_max_warps();
+int multi_warp_ctas_per_sm();
+int multi_warp_head(int nsmpl, int nwarp, size_t smem_per_cta);
+size_t multi_warp_tail_bytes(int nsmpl, int head);
+cudaError_t launch_multi_warp_kernel(const KArgs &a, int grid, int nwarp, int head, uint8_t *tail, cudaStream_t st);
 /*  warp-per-site kernel for grouped calling (-G) of two-allele sites (mcall_biallelic_groups.cu)  */
 bool biallelic_groups_ok(int nsmpl, int ngroups);
 int biallelic_groups_warps();

@@ -146,7 +146,7 @@ static __device__ __noinline__ void mm_epilogue(MMShared<NALS,BLOCK> *shp, const
     }
     const int nesc_raw = sh.nesc;
     const int s = lane < min(nesc_raw, MM_ESC_CAP) ? sh.esc[lane] : 0;
-    mm_decide<NALS,12>(&sh, su, a, lane, pl2p_s, pack_s, nesc_raw, s, sh.esc_pl[lane], sums_g + s, tl, n0, ps);
+    mm_decide<NALS,12>(&sh, su, a, lane, pl2p_s, pack_s + (uint32_t)(s*MMGeom<NALS>::RS), nesc_raw, sh.esc_pl[lane], sums_g + s, tl, n0, ps);
     if ( lane==0 ) sh.nesc = 0;
 }
 

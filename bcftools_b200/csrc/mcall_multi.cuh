@@ -1,5 +1,6 @@
 /*  mcall_multi.cuh -- what the site kernels of the multi-allelic classes share: the CTA-per-site kernel of the 3-5 allele
- *  classes (mcall_multi.cu) and the warp-per-site kernel of the 3-allele class (mcall_triallelic.cu).  Per-site set-up, the
+ *  classes (mcall_multi.cu) and the warp-per-site kernels of the 3-allele class (mcall_triallelic.cu) and of the 4-allele
+ *  class (mcall_multi_warp.cu).  Per-site set-up, the
  *  general path of a sample with missing values, the allele-set decision and the site record, and the literal FP64 calls of
  *  phase 2.  A kernel keeps its decision record in a struct of its own; the templates below read and write it by member name.  */
 #pragma once
@@ -48,6 +49,12 @@ __device__ __forceinline__ void mm_stg128(void *p, int x, int y, int z, int w)
 __device__ __forceinline__ void mm_stg64(void *p, int x, int y) { asm volatile("st.global.cs.v2.s32 [%0], {%1,%2};" :: "l"(p), "r"(x), "r"(y) : "memory"); }
 __device__ __forceinline__ void mm_stg32(void *p, int x) { asm volatile("st.global.cs.s32 [%0], %1;" :: "l"(p), "r"(x) : "memory"); }
 __device__ __forceinline__ uint32_t mm_pack4(int a, int b, int c, int d) { return (uint32_t)a | (uint32_t)b<<8 | (uint32_t)c<<16 | (uint32_t)d<<24; }
+/*  byte j of a packed row: a 32-bit shared address, or a generic pointer (the warp kernel of the 4-allele class keeps part
+ *  of its packed copy in global memory)  */
+__device__ __forceinline__ uint32_t mm_row_u8(uint32_t row_s, uint32_t j) { return mm_ldsu8(row_s + j); }
+__device__ __forceinline__ uint32_t mm_row_u8(const uint8_t *row, uint32_t j) { return row[j]; }
+__device__ __forceinline__ void mm_row_st8(uint32_t row_s, uint32_t j, uint32_t v) { asm volatile("st.shared.u8 [%0], %1;" :: "r"(row_s + j), "r"(v) : "memory"); }
+__device__ __forceinline__ void mm_row_st8(uint8_t *row, uint32_t j, uint32_t v) { row[j] = (uint8_t)v; }
 
 static __device__ __noinline__ double mm_log(double x) { return log(x); }
 static __device__ __noinline__ double mm_exp(double x) { return exp(x); }
@@ -95,8 +102,8 @@ template<int NALS> struct MMSlow
  *  sum_g != nullptr, the normaliser), so that phase 2 treats it like any other sample.  No data: packed zeros; sum = -1 when
  *  the row still holds sentinels (phase 2 then re-derives the output row from the int32 values), +G otherwise.
  *  Returns "the row still holds sentinels and carries no data".  */
-template<int NALS>
-static __device__ __noinline__ bool mm_slow_sample(const int *row, const MMSetup<NALS> *su, uint32_t pl2p_s, uint32_t row_s, double *sum_g, MMSlow<NALS> *acc)
+template<int NALS, class RowT>
+static __device__ __noinline__ bool mm_slow_sample(const int *row, const MMSetup<NALS> *su, uint32_t pl2p_s, RowT dst, double *sum_g, MMSlow<NALS> *acc)
 {
     using S = Shape<NALS>;
     constexpr int G = S::G, RS = MMGeom<NALS>::RS;
@@ -145,8 +152,7 @@ static __device__ __noinline__ bool mm_slow_sample(const int *row, const MMSetup
                         acc->lk[k] += mm_log(val);
                     }
     }
-    for (int j=0; j<RS; j++)
-        asm volatile("st.shared.u8 [%0], %1;" :: "r"(row_s + (uint32_t)j), "r"((data && j<G) ? pl[j] : 0) : "memory");
+    for (int j=0; j<RS; j++) mm_row_st8(dst, (uint32_t)j, (data && j<G) ? (uint32_t)pl[j] : 0u);
     if ( sum_g ) asm volatile("st.global.cg.L2::cache_hint.f64 [%0], %1, %2;" :: "l"(sum_g), "d"(sum), "l"(mm_policy_evict_last()) : "memory");
     return raw;
 }
@@ -283,14 +289,15 @@ static __device__ __noinline__ void mm_finalize(Rec *shp, const KArgs &a)
  *  QUAL candidates, trimming maps and the phase-2 constants, written to the kernel's record `sh`.  From the main loop:
  *  tl = log of the product over its samples of the lane's allele set (lanes NALS.. with a live set) or of the normalisers
  *  (lane 31), n0 = the samples that went through it without data, ps = sum of PL[lane/lane] (lanes < NALS).
- *  ACB: bits per allele of the AC increments in slot_out.  Returns "the lane's listed sample holds sentinels and no data".  */
-template<int NALS, int ACB, class Rec>
-static __device__ __noinline__ bool mm_decide(Rec *shp, const MMSetup<NALS> *su, const KArgs &a, int lane, uint32_t pl2p_s, uint32_t pack_s,
-                                              int nesc_raw, int esc_s, const int *esc_row, double *esc_sum, double tl, int n0, long long ps)
+ *  esc_dst: the packed row of the lane's listed sample.  ACB: bits per allele of the AC increments in slot_out.
+ *  Returns "the lane's listed sample holds sentinels and no data".  */
+template<int NALS, int ACB, class Rec, class RowT>
+static __device__ __noinline__ bool mm_decide(Rec *shp, const MMSetup<NALS> *su, const KArgs &a, int lane, uint32_t pl2p_s, RowT esc_dst,
+                                              int nesc_raw, const int *esc_row, double *esc_sum, double tl, int n0, long long ps)
 {
     using S = Shape<NALS>;
     using GE = MMGeom<NALS>;
-    constexpr int G = S::G, NPAIR = S::NPAIR, NSUB = S::NSUB, NSET = GE::NSET, RS = GE::RS;
+    constexpr int G = S::G, NPAIR = S::NPAIR, NSUB = S::NSUB, NSET = GE::NSET;
     constexpr double LN10_10 = 0.2302585092994045684017991454684;
     constexpr double LOG_G = G==6 ? 1.791759469228055000812477358381 : (G==10 ? 2.302585092994045684017991454684 : 2.708050201102210065996004570148);   /* ln 6, ln 10, ln 15 */
     Rec &sh = *shp;
@@ -305,7 +312,7 @@ static __device__ __noinline__ bool mm_decide(Rec *shp, const MMSetup<NALS> *su,
     bool raw = false;
     const int nesc = min(nesc_raw, MM_ESC_CAP);
     if ( nesc_raw > MM_ESC_CAP ) sl.punt = 1;
-    else if ( lane < nesc ) raw = mm_slow_sample<NALS>(esc_row, su, pl2p_s, pack_s + (uint32_t)(esc_s*RS), esc_sum, &sl);
+    else if ( lane < nesc ) raw = mm_slow_sample<NALS>(esc_row, su, pl2p_s, esc_dst, esc_sum, &sl);
     if ( __any_sync(0xffffffffu, nesc>0) )
     {
         #pragma unroll 1
@@ -519,12 +526,13 @@ static __device__ __noinline__ int mm_fast2_exact(uint32_t a, uint32_t b, uint32
     fast2_call(lds64c(pl2p_s + 8u*a), lds64c(pl2p_s + 8u*b), lds64c(pl2p_s + 8u*c), sum, q0, q1, __dmul_rn(2.0, q1), thr_s, k, g);
     return k | g<<8;
 }
-static __device__ __noinline__ int mm_fast3_exact(uint32_t row_s, uint32_t jgt_s, double sum, uint32_t q_s, uint32_t pl2p_s, uint32_t thr_s)
+template<class RowT>
+static __device__ __noinline__ int mm_fast3_exact(RowT row, uint32_t jgt_s, double sum, uint32_t q_s, uint32_t pl2p_s, uint32_t thr_s)
 {
     const double q0 = lds64(q_s), q1 = lds64(q_s + 8u), q2 = lds64(q_s + 16u);
     double p[6];
     #pragma unroll
-    for (int k=0; k<6; k++) p[k] = lds64c(pl2p_s + 8u*mm_ldsu8(row_s + (uint32_t)lds32(jgt_s + 4u*k)));
+    for (int k=0; k<6; k++) p[k] = lds64c(pl2p_s + 8u*mm_row_u8(row, (uint32_t)lds32(jgt_s + 4u*k)));
     int k, g;
     fast3_call(p, sum, q0, q1, q2, __dmul_rn(2.0, q1), __dmul_rn(2.0, q2), thr_s, k, g);
     return k | g<<8;

@@ -234,7 +234,7 @@ __global__ void __launch_bounds__(TW_MAXWARP*32, TW_MINCTA) mcall_triallelic_war
         __syncwarp();               /* the list and the packed rows of every lane are visible */
         const int nesc_raw = rec.nesc;
         const int my_esc = lane < min(nesc_raw, MM_ESC_CAP) ? (int)rec.esc[lane] : 0;
-        const bool my_raw = mm_decide<3,16>(&rec, &su, a, lane, pl2p_s, pack_s, nesc_raw, my_esc, site_pl + (size_t)my_esc*G, nullptr, tl, n0, ps);
+        const bool my_raw = mm_decide<3,16>(&rec, &su, a, lane, pl2p_s, pack_s + (uint32_t)(my_esc*6), nesc_raw, site_pl + (size_t)my_esc*G, nullptr, tl, n0, ps);
         __syncwarp();
 
         /* the next site is claimed now: the atomic's latency hides behind phase 2.  Its set-up (site_list, then qs / pl_off /
