@@ -94,6 +94,7 @@ struct mcb_ctx
     int64_t opt_block_c[NCLASS] = {0,0,0,0,0,0};        /* per class override of the CTA size */
     int64_t opt_tile_bytes_c[NCLASS] = {0,0,0,0,0,0};   /* per class override of tile_bytes */
     int64_t opt_bps_c[NCLASS] = {0,0,0,0,0,0};          /* per class cap of resident CTAs per SM (0 = as many as fit): lets classes share an SM */
+    int64_t opt_max_ctas = 0;            /* cap of every persistent launch grid (0 = none): a worker calls many sites of a small batch */
     cudaStream_t cstream[NCLASS] = {};   /* one stream per allele-count class: their persistent grids overlap */
     cudaEvent_t  cev_fork = nullptr, cev_join[NCLASS] = {};
     cudaEvent_t kev[NCLASS+1] = {};      /* events around the per-class launches (time_kernels=1) */
@@ -190,6 +191,7 @@ extern "C" int mcb_set_option(mcb_ctx *ctx, const char *key, int64_t value)
     else if ( !strcmp(key,"order") )         ctx->opt_order = value;
     else if ( !strcmp(key,"multi") )         ctx->opt_multi = value;
     else if ( !strcmp(key,"bgroups") )       ctx->opt_bgroups = value;
+    else if ( !strcmp(key,"max_ctas") )      { if ( value<0 ) return MCB_EINVAL; ctx->opt_max_ctas = value; }
     else if ( !strcmp(key,"gorder") )
     {
         int seen = 0; int64_t v = value;
@@ -410,6 +412,13 @@ extern "C" int mcb_selftest_div(mcb_ctx *ctx, int mode, uint64_t n, uint64_t see
 }
 
 /* ---- launch geometry -------------------------------------------------------------------------------- */
+/*  The grid a persistent kernel is launched with: `grid`, capped by option max_ctas.  Only the launch sees the cap; kernel choice
+ *  and scratch sizing use the uncapped grid, so a capped call runs the kernels of an uncapped one with many sites per worker.  */
+static inline int launch_grid(const mcb_ctx *ctx, int grid)
+{
+    return ctx->opt_max_ctas > 0 ? (int)std::min<int64_t>(grid, ctx->opt_max_ctas) : grid;
+}
+
 /*  CTA size, tile size and ring size per allele-count class.  Explicit options win; the defaults below are the best
  *  settings of the sweeps in profiles/ (measured at 2,504 samples) plus smaller CTAs for small sample counts, where a
  *  128-thread CTA would have mostly idle lanes.                                                                    */
@@ -472,7 +481,7 @@ static int enqueue_class0(mcb_ctx *ctx, KArgs &a, const mcb_batch *b, const mcb_
     }
     a.site_list = lists; a.site_count = counts;
     a.grp_off = ctx->d_grp_off; a.grp_smpl = ctx->d_grp_smpl; a.smpl2grp = ctx->d_smpl2grp; a.ngroups = ctx->ngroups;
-    CK(launch_generic_kernel(a, sc.gen_grp, sc.gen_pl, sc.gen_sum, std::min(sc.gen_grid, std::max(1, b->nsites)), st));
+    CK(launch_generic_kernel(a, sc.gen_grp, sc.gen_pl, sc.gen_sum, launch_grid(ctx, std::min(sc.gen_grid, std::max(1, b->nsites))), st));
     return MCB_OK;
 }
 
@@ -519,14 +528,14 @@ static int enqueue_adjudication(mcb_ctx *ctx, const KArgs &a1, const mcb_batch *
     {
         a.site_list = lists + (size_t)nals*list_stride; a.site_count = counts + nals;
         a.work_counter = counts + NCLASS + nals;
-        if ( ctx->ngroups > 1 ) { CK(launch_groups_kernel(nals, a, (char*)sc.grp + (size_t)(nals-1)*gper_class, ggrid, st)); continue; }
+        if ( ctx->ngroups > 1 ) { CK(launch_groups_kernel(nals, a, (char*)sc.grp + (size_t)(nals-1)*gper_class, launch_grid(ctx, ggrid), st)); continue; }
         size_t ring; tile_geometry(ctx, nals, pl_es, &a.tile_smpl, &a.nstage, &ring);
         const int block = (pl_es==2 || gpk) ? 128 : class_block(ctx, nals);
         int nb = 1;
         CK(site_kernel_occupancy(nals, ploidy, gpk, block, pl_es, ring, &nb));
         if ( nb<1 ) return cuda_fail(ctx, cudaErrorLaunchOutOfResources, "site kernel does not fit on an SM");
         const int grid = (int)std::min<int64_t>((int64_t)b->nsites, (int64_t)ctx->nsm*nb);
-        cudaError_t le = launch_site_kernel(nals, ploidy, gpk, block, pl_es, a, grid, ring, st);
+        cudaError_t le = launch_site_kernel(nals, ploidy, gpk, block, pl_es, a, launch_grid(ctx, grid), ring, st);
         if ( le!=cudaSuccess ) return cuda_fail(ctx, le, "near-tie adjudication: site kernel");
     }
     if ( ctx->p.max_nals > 5 && pl_es == 4 )        /* 6..32 alleles (class 0) */
@@ -609,12 +618,12 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
                 ab.fb_count = counts + NCLASS + 8 + nals;
                 const int w = biallelic_groups_warps();
                 const int bgrid = (int)std::min<int64_t>(((int64_t)b->nsites + w - 1)/w, (int64_t)ctx->nsm*biallelic_groups_ctas_per_sm());
-                cudaError_t le = launch_biallelic_groups_kernel(ab, std::max(1, bgrid), cs);
+                cudaError_t le = launch_biallelic_groups_kernel(ab, launch_grid(ctx, std::max(1, bgrid)), cs);
                 if ( le!=cudaSuccess ) return cuda_fail(ctx, le, "two-allele grouped kernel");
                 launches++;
                 a.site_list = ab.fb_list; a.site_count = ab.fb_count;
             }
-            CK(launch_groups_kernel(nals, a, (char*)sc.grp + (size_t)(nals-1)*per_class, grid, cs));
+            CK(launch_groups_kernel(nals, a, (char*)sc.grp + (size_t)(nals-1)*per_class, launch_grid(ctx, grid), cs));
             if ( gfork ) { CK(cudaEventRecord(ctx->cev_join[nals], cs)); CK(cudaStreamWaitEvent(st, ctx->cev_join[nals], 0)); }
             if ( gtiming ) CK(cudaEventRecord(ctx->kev[nals], st));
             launches++;
@@ -673,6 +682,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
             int grid = (int)std::min<int64_t>(((int64_t)b->nsites + bw_warps - 1)/bw_warps, (int64_t)ctx->nsm*biallelic_ctas_per_sm());
             if ( ctx->opt_blocks_per_sm>0 ) grid = std::min<int>(grid, ctx->nsm*(int)std::min<int64_t>(biallelic_ctas_per_sm(), ctx->opt_blocks_per_sm));
             if ( ctx->opt_bps_c[2]>0 ) grid = std::min<int>(grid, ctx->nsm*(int)std::min<int64_t>(biallelic_ctas_per_sm(), ctx->opt_bps_c[2]));
+            grid = launch_grid(ctx, grid);
             cudaStream_t cs = fork ? ctx->cstream[nals] : st;
             if ( fork ) CK(cudaStreamWaitEvent(cs, ctx->cev_fork, 0));
             cudaError_t le = launch_biallelic_warp_kernel(a, ploidy, grid, bw_warps, cs);
@@ -730,7 +740,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
         }
         if ( tw_warps )
         {
-            const int tgrid = (int)std::min<int64_t>(((int64_t)b->nsites + tw_warps - 1)/tw_warps, (int64_t)ctx->nsm*triallelic_ctas_per_sm());
+            const int tgrid = launch_grid(ctx, (int)std::min<int64_t>(((int64_t)b->nsites + tw_warps - 1)/tw_warps, (int64_t)ctx->nsm*triallelic_ctas_per_sm()));
             KArgs am = a;
             am.fb_list = lists + (size_t)(NCLASS + nals)*list_stride;
             am.fb_count = counts + NCLASS + 8 + nals;
@@ -751,7 +761,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
         else if ( mw_warps )
         {
             const int ncta = multi_warp_ctas_per_sm();
-            const int mgrid = (int)std::min<int64_t>(((int64_t)b->nsites + mw_warps - 1)/mw_warps, (int64_t)ctx->nsm*ncta);
+            const int mgrid = launch_grid(ctx, (int)std::min<int64_t>(((int64_t)b->nsites + mw_warps - 1)/mw_warps, (int64_t)ctx->nsm*ncta));
             const size_t tail = multi_warp_tail_bytes(a.nsmpl, mw_head);
             if ( tail && (size_t)ctx->nsm*ncta*mw_warps*tail > sc.mw_tail_bytes[nals] )
             {
@@ -810,7 +820,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
                     am.mm_sums = sc.mm_sums[nals];
                     am.fb_list = lists + (size_t)(NCLASS + nals)*list_stride;
                     am.fb_count = counts + NCLASS + 8 + nals;
-                    cudaError_t le = launch_multi_kernel(nals, mblock, am, mgrid, cs);
+                    cudaError_t le = launch_multi_kernel(nals, mblock, am, launch_grid(ctx, mgrid), cs);
                     if ( le==cudaSuccess && getenv("MCB_DEBUG_SYNC") ) le = cudaStreamSynchronize(cs);
                     if ( le!=cudaSuccess )
                     {
@@ -827,6 +837,7 @@ static int enqueue(mcb_ctx *ctx, const mcb_batch *b, const mcb_result *r, int32_
             }
         }
         {
+            grid = launch_grid(ctx, grid);
             cudaError_t le = launch_site_kernel(nals, ploidy, gpk, block, pl_es, a, grid, ring, cs);
             if ( le==cudaSuccess && getenv("MCB_DEBUG_SYNC") ) le = cudaStreamSynchronize(cs);
             if ( le!=cudaSuccess )

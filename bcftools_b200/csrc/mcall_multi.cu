@@ -144,9 +144,26 @@ static __device__ __noinline__ void mm_epilogue(MMShared<NALS,BLOCK> *shp, const
         #pragma unroll
         for (int w=0; w<NW; w++) ps += sh.red_pls[w][lane];
     }
-    const int nesc_raw = sh.nesc;
-    const int s = lane < min(nesc_raw, MM_ESC_CAP) ? sh.esc[lane] : 0;
-    mm_decide<NALS,12>(&sh, su, a, lane, pl2p_s, pack_s + (uint32_t)(s*MMGeom<NALS>::RS), nesc_raw, sh.esc_pl[lane], sums_g + s, tl, n0, ps);
+    const int nesc_raw = sh.nesc, nesc = min(nesc_raw, MM_ESC_CAP);
+    /* every warp's lanes append to the list through one atomic counter, so its order follows warp scheduling; mm_decide adds
+       the lanes' FP64 terms in lane order, so lane r takes the entry of rank r by sample index (the samples are distinct):
+       a bitonic sort over the warp of (sample << 5 | list position), unused positions last */
+    int src = lane;
+    if ( nesc > 1 && nesc_raw <= MM_ESC_CAP )
+    {
+        int v = ((lane < nesc ? (int)sh.esc[lane] : 0x1ffff) << 5) | lane;
+        #pragma unroll
+        for (int k=2; k<=32; k<<=1)
+            #pragma unroll
+            for (int j=k>>1; j>0; j>>=1)
+            {
+                const int o = __shfl_xor_sync(0xffffffffu, v, j);
+                v = (((lane & j) == 0) == ((lane & k) == 0)) ? min(v, o) : max(v, o);
+            }
+        src = v & 31;
+    }
+    const int s = lane < nesc ? sh.esc[src] : 0;
+    mm_decide<NALS,12>(&sh, su, a, lane, pl2p_s, pack_s + (uint32_t)(s*MMGeom<NALS>::RS), nesc_raw, sh.esc_pl[src], sums_g + s, tl, n0, ps);
     if ( lane==0 ) sh.nesc = 0;
 }
 

@@ -192,7 +192,9 @@ int   mcb_get_stats(const mcb_ctx *ctx, int64_t stats[4]);
  *  sample-sequential sums of logs of mcall_find_best_alleles (mcall.c:591-710).  All of the site's outputs are overwritten
  *  by that evaluation and it carries MCB_SITE_NEAR_TIE | MCB_SITE_ADJUDICATED.  Needs result.site_flags: a call without it
  *  returns MCB_EINVAL.  Compacted PL output (pl_off_out) stays within the documented capacity: a flagged site reserves the
- *  block of its full genotype count.  "exact_phase1" (0|1): every site through the literal phase 1.  */
+ *  block of its full genotype count.  "exact_phase1" (0|1): every site through the literal phase 1.
+ *  "max_ctas" (>= 0, default 0 = no cap): every persistent kernel is launched with at most that many CTAs, so that each warp or
+ *  CTA calls many sites of a small batch; which kernels run and how their scratch is sized do not change.  A test hook.  */
 int   mcb_set_option(mcb_ctx *ctx, const char *key, int64_t value);
 int   mcb_version(void);
 /*  device milliseconds of the site kernel per allele-count class (ms[1..5], ms[0]=sum) of the last
